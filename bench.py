@@ -50,6 +50,7 @@ WORKLOADS = {
 EPISODE_LEN = 1000
 TABLE_ROWS = 4096
 L2_BYTES = 126e6
+DUMP_BYTES = 60 << 20                                         # --dump-outputs: under 64 MB with the .npy headers
 
 
 def algorithmic_bytes_per_asset_step(A, W, F, commission, obs, sinks=0.0):
@@ -70,6 +71,23 @@ def ncu_traffic_bytes(workload):
             return json.load(fh).get(workload, {}).get("dram_bytes_per_launch")
     except Exception:
         return None
+
+
+def dump_outputs(out_dir, arrays, E, limit=DUMP_BYTES):
+    """Writes `arrays` (name -> (tensor, env axis)) as out_dir/<name>.npy, float32 (int64 as float64, exact).  While
+    they fit in `limit` bytes they go out whole; otherwise every array is cut to the same fixed, seeded sample of envs,
+    in ascending order, and env_index.npy lists them."""
+    import numpy as np
+    import torch
+    per_env = sum(4 * t.numel() // E for t, _ in arrays.values())
+    if per_env * E > limit:
+        idx = torch.randperm(E, generator=torch.Generator().manual_seed(0))[:limit // (per_env + 8)].sort().values
+        arrays = {k: (t.index_select(ax, idx.to(t.device)), ax) for k, (t, ax) in arrays.items()}
+        arrays["env_index"] = (idx, 0)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (t, _) in arrays.items():
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype == np.int64 else np.float32))
 
 
 def measured_peak_gbs():
@@ -582,7 +600,13 @@ def main():
                     help="state-only workloads: advance K steps per launch through pmrl_env_step_burst (imagination bursts)")
     ap.add_argument("--tune", action="append", default=[], metavar="KEY=VAL",
                     help="kernel launch-shape override: group|ctas|fast|rt|staged = int (pmrl_set_tuning)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last one returned (obs, reward, done; rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -629,10 +653,12 @@ def main():
     stats_in_sync = None
 
     graph_launches_per_step = 0
-    burst = max(1, args.graph)
+    burst = max(1, args.graph or args.burst)
+    if args.steps % burst:
+        raise SystemExit(f"--steps must be a multiple of the {burst}-step burst")
+    returned = [None]                                         # what the last timed step returned (--dump-outputs)
     if args.graph:
-        if args.steps % burst or args.warmup % burst:
-            args.steps = max(burst, args.steps // burst * burst)
+        if args.warmup % burst:
             args.warmup = max(burst, -(-args.warmup // burst) * burst)
         c0 = ctx.lib.pmrl_launch_count()
         static_actions, replay = env.graphed_step(obs=obs, steps=burst)
@@ -642,12 +668,10 @@ def main():
         def one_step(i):                                      # called once per env step; a burst is replayed on its first step
             if i % burst == 0:
                 static_actions.copy_(burst_pool[(i // burst) % n_pool])   # the policy would write its actions here
-                replay()
+                returned[0] = replay()
     elif args.burst:
-        burst = args.burst
         if obs:
             raise SystemExit("--burst is a state-only mode")
-        args.steps = max(burst, args.steps // burst * burst)
         args.warmup = max(burst, -(-args.warmup // burst) * burst)
         burst_pool = [torch.stack([pool[(j + k) % n_pool] for k in range(burst)]) for j in range(n_pool)]
         b_rew = torch.empty(burst, E, dtype=torch.float32, device=dev)
@@ -655,10 +679,10 @@ def main():
 
         def one_step(i):
             if i % burst == 0:
-                env.step_burst(burst_pool[(i // burst) % n_pool], b_rew, b_done)
+                returned[0] = env.step_burst(burst_pool[(i // burst) % n_pool], b_rew, b_done)
     else:
         def one_step(i):
-            env.step(pool[i % n_pool], obs=obs)
+            returned[0] = env.step(pool[i % n_pool], obs=obs)
             if reducer is not None and i % args.stats_every == 0:
                 reducer.launch(env._stats)
 
@@ -670,6 +694,12 @@ def main():
     if args.graph:
         gpu_launches = graph_launches_per_step * args.steps      # replayed from the graph: counted at capture time
     clocks = sampler.summary() if rank == 0 else None
+    if args.dump_outputs and rank == 0:                       # before anything else reuses the env's output buffers
+        *o, rew, done = returned[0]                           # (obs | None, reward, done) or, from a burst, (reward, done)
+        outs = {"reward": (rew, rew.dim() - 1), "done": (done, done.dim() - 1)}
+        if o and o[0] is not None:
+            outs["obs"] = (o[0], 0)
+        dump_outputs(args.dump_outputs, outs, E)
     if reducer is not None:                                   # the last step's reduced vector must equal a fresh reduce
         last = reducer.result()
         fresh = pdist.all_reduce_stats(env._stats.clone())

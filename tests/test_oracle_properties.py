@@ -1,12 +1,13 @@
 """Property tests of the restated oracle (hypothesis; CPU): invariants the reference transition must keep."""
 import numpy as np
-from hypothesis import given, settings, strategies as st
+from hypothesis import example, given, settings, strategies as st
 
 from oracle.env_oracle import OracleEnv, commission_mu, normalise_actions
 
 
 @settings(max_examples=40, deadline=None)
 @given(st.integers(2, 40), st.integers(2, 12), st.integers(0, 2 ** 31 - 1), st.sampled_from([0.0, 0.0025, 0.01]))
+@example(A=8, W=2, seed=489224, c=0.0)                          # draws a signed row that sums to 1 at step 4
 def test_transition_invariants(A, W, seed, c):
     rs = np.random.RandomState(seed)
     E, S = 5, 3 * W
@@ -14,6 +15,8 @@ def test_transition_invariants(A, W, seed, c):
     for s in range(S):
         act = rs.standard_normal((E, A)).astype(np.float32)
         act[:, 0] = -np.abs(act[:, 0]) - 0.1                    # a negative entry: softmax branch → the target is a simplex
+        # ... unless the row also sums to 1 (trading_env.py:58 keeps such a row as is): move those sums away from 1
+        act[:, 0] -= np.where(np.abs(act.sum(1) - 1) < 1e-3, np.float32(1), np.float32(0))
         y = (1 + 0.02 * rs.standard_normal((E, A))).astype(np.float32); y[:, 0] = 1
         v_prev = env.value.copy()
         idx_prev = env.idx.copy()
