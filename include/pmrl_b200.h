@@ -41,7 +41,8 @@
  *   idx      [E] i32       ring write pointer;  is_full [E] u8;  t [E] i32 local step k
  *   t0       [E] i32       episode offset: at local step k the env sees table rows
  *                          [t0+k, t0+k+W) and the price relative of row t0+k+W-1
- *   obs      [E, A, W, F]  reference observation layout (net/lsre_cann.py:105)
+ *   obs      [E, A, W, F]  reference observation layout (net/lsre_cann.py:105); fp32, or bf16 bit patterns with
+ *                          PMRL_OBS_BF16 (everything else stays fp32)
  */
 #ifndef PMRL_B200_H
 #define PMRL_B200_H
@@ -75,6 +76,14 @@ extern "C" {
 #define PMRL_OBS_NONE    0   /* state-only step ("Mode S") */
 #define PMRL_OBS_FULL    1   /* gather feature window + weight channel into obs ("Mode O") */
 #define PMRL_OBS_WEIGHTS 2   /* overwrite only channel F-1 of a caller-filled obs (compat shim; trading_env.py:103) */
+#define PMRL_OBS_BF16    0x100  /* OR-ed into PMRL_OBS_FULL only (pmrl_env_reset, pmrl_env_step, PmrlStepIO.obs_mode,
+                                   pmrl_env_step_host, pmrl_obs_build): the `float* obs` argument then points to [E, A, W, F]
+                                   uint16_t bf16 bit patterns, each the round-to-nearest-even (cvt.rn.bf16.f32) of the fp32 value
+                                   the plain FULL mode writes; half the obs bytes.  State, tables, reward, done, stats and sinks
+                                   stay fp32 and bit-identical to an fp32 run.  Accepted for exactly the shapes FULL accepts;
+                                   WEIGHTS | BF16, NONE | BF16 and unknown bits fail with PMRL_E_ARG before any launch.  A library
+                                   built before this flag rejects it with "bad obs_mode" (PMRL_E_ARG): that is how a binding
+                                   detects support (PMRL_ABI_VERSION is unchanged). */
 
 typedef struct PmrlEnvCfg {
     int32_t E, A, W, F;        /* envs on this device, assets, window, obs channels (weight slot = F-1) */
@@ -330,6 +339,21 @@ int pmrl_rollout_gather_index(int32_t S, int32_t E, int32_t A, int32_t W, int32_
                               float* s_out, float* a_out, float* r_out, float* pv_out, float* pa_out, float* p_out,
                               void* stream);
 
+/* The two rollout gathers for a buffer whose observations are bf16 (PMRL_OBS_BF16): the same parameters, but s (full mode)
+ * and s_out are uint16_t bf16 bit patterns; the regenerated obs of the index-mode gather is rounded from the fp32 values like
+ * the step kernels round theirs.  The other outputs stay fp32. */
+int pmrl_rollout_gather_bf16(int32_t S, int32_t E, int32_t A, int32_t W, int32_t F, int32_t B,
+                             const int32_t* slots, const int32_t* envs,
+                             const uint16_t* s, const float* a, const float* v, const float* r, const float* y,
+                             uint16_t* s_out, float* a_out, float* r_out, float* pv_out, float* pa_out, float* p_out,
+                             void* stream);
+int pmrl_rollout_gather_index_bf16(int32_t S, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
+                                   const int32_t* slots, const int32_t* envs,
+                                   const int32_t* bi, const float* a, const float* v, const float* r,
+                                   const float* wp, const float* feat_am, const float* y_tm,
+                                   uint16_t* s_out, float* a_out, float* r_out, float* pv_out, float* pa_out, float* p_out,
+                                   void* stream);
+
 /* Off-policy index replay: store (i, a, r) of all E envs at [epoch_slot, step_slot] (buffer.py:31-37).
  * Buffers: bi [P, L, E] i32, ba [P, L, E, A], br [P, L, E]. */
 int pmrl_replay_add(int32_t P, int32_t L, int32_t E, int32_t A, int32_t epoch_slot, int32_t step_slot,
@@ -344,6 +368,11 @@ int pmrl_replay_gather(int32_t P, int32_t L, int32_t E, int32_t A, int32_t W, in
                        const int32_t* epochs, const int32_t* envs, const int32_t* starts,
                        const int32_t* bi, const float* ba, const float* br, const float* feat_am,
                        float* s_out, float* a_out, float* r_out, float* s2_out, void* stream);
+/* The same sample with s_out / s2_out as uint16_t bf16 bit patterns (PMRL_OBS_BF16 rounding); a_out, r_out stay fp32. */
+int pmrl_replay_gather_bf16(int32_t P, int32_t L, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
+                            const int32_t* epochs, const int32_t* envs, const int32_t* starts,
+                            const int32_t* bi, const float* ba, const float* br, const float* feat_am,
+                            uint16_t* s_out, float* a_out, float* r_out, uint16_t* s2_out, void* stream);
 
 /* ---- differentiable batched reward (agent/pg/pg.py:40-82) ---- */
 

@@ -15,6 +15,14 @@ import torch
 
 from . import _lib
 
+_OBS_DTYPES = {"float32": torch.float32, "bfloat16": torch.bfloat16}
+
+
+def _obs_dtype(name):
+    if name not in _OBS_DTYPES:
+        raise ValueError(f"unknown obs_dtype {name!r}; expected one of {tuple(_OBS_DTYPES)}")
+    return _OBS_DTYPES[name]
+
 
 class DeviceRolloutBuffer:
     """On-policy epoch buffer (replay/rollout_buffer.py:7-142) batched over E envs, in one of two storage modes:
@@ -30,17 +38,22 @@ class DeviceRolloutBuffer:
     Either way the rows of a slot are written by the step kernel itself: `sinks(step)` returns the keyword arguments for
     `BatchedTradingEnv.step_io` (reward → r[slot], action_sink → a[slot], value_sink → v[slot], obs out → s[slot + 1], …),
     so no copy kernel runs per step.  `add` keeps the reference's call (rollout_buffer.py:43-57) for callers that have
-    the rows elsewhere."""
+    the rows elsewhere.
+
+    obs_dtype="bfloat16": s is stored (full mode) and returned by `gather` / `sample` / `sample_random` (both modes) as
+    bf16, half the bytes; the env feeding it must have the same obs_dtype.  a, v, r, prices stay fp32."""
 
     def __init__(self, num_features: int, train_len: int, num_envs: int, num_assets: int, window_size: int,
                  initial_cash: float = 25000.0, batch_size: int = 64, device=None, store_obs: bool = True,
-                 mode: str = "full", feat_am=None, y_tm=None):
+                 mode: str = "full", feat_am=None, y_tm=None, obs_dtype: str = "float32"):
         if not torch.cuda.is_available():
             raise _lib.PmrlError("DeviceRolloutBuffer needs a CUDA device (pmrl_b200 has no CPU fallback)")
         if mode not in ("full", "index"):
             raise ValueError("mode must be 'full' or 'index'")
         self.lib = _lib.load()
         self.mode = mode
+        self.obs_dtype = _obs_dtype(obs_dtype)
+        self._bf16 = self.obs_dtype is torch.bfloat16
         self.F, self.E, self.A, self.W = num_features, num_envs, num_assets, window_size
         self.step_offset = window_size - 1                      # rollout_buffer.py:10
         self.epoch_len = train_len - self.step_offset           # rollout_buffer.py:11
@@ -53,7 +66,7 @@ class DeviceRolloutBuffer:
         self.s = self.y = self.bi = self.wp = None
         self.feat_am, self.y_tm = feat_am, y_tm
         if mode == "full":
-            self.s = torch.zeros(S, E, A, W, F, device=dev) if store_obs else None
+            self.s = torch.zeros(S, E, A, W, F, dtype=self.obs_dtype, device=dev) if store_obs else None
             self.y = torch.zeros(S, E, A, device=dev)           # `prices` (rollout_buffer.py:12), filled by set_prices/add
         else:
             if feat_am is None or y_tm is None:
@@ -139,7 +152,10 @@ class DeviceRolloutBuffer:
             r2 = r.reshape(self.E).to(torch.float32).contiguous()
             s2 = None
             if s is not None and self.s is not None and s.data_ptr() != self.s[slot].data_ptr():
-                s2 = s.reshape(self.E, self.A, self.W, self.F).to(torch.float32).contiguous()
+                if self._bf16:                                  # converting copy into the bf16 slot (round to nearest even)
+                    self.s[slot].copy_(s.reshape(self.E, self.A, self.W, self.F))
+                else:
+                    s2 = s.reshape(self.E, self.A, self.W, self.F).to(torch.float32).contiguous()
             rc = self.lib.pmrl_rollout_add(self.E, self.A, self.W, self.F, slot, _lib.ptr(s2), _lib.ptr(a2), _lib.ptr(v2),
                                            _lib.ptr(r2), _lib.ptr(self.s), _lib.ptr(self.a), _lib.ptr(self.v),
                                            _lib.ptr(self.r), _lib.current_stream())
@@ -164,10 +180,12 @@ class DeviceRolloutBuffer:
         envs = torch.as_tensor(envs).to(self.device, torch.int32).contiguous()
         B = slots.numel()
         A, W, F, dev = self.A, self.W, self.F, self.device
-        s = torch.empty(B, A, W, F, device=dev); a = torch.empty(B, A, 1, device=dev); r = torch.empty(B, 1, 1, device=dev)
+        s = torch.empty(B, A, W, F, dtype=self.obs_dtype, device=dev)
+        a = torch.empty(B, A, 1, device=dev); r = torch.empty(B, 1, 1, device=dev)
         pv = torch.empty(B, 1, 1, device=dev); pa = torch.empty(B, A, 1, device=dev); p = torch.empty(B, A, 1, device=dev)
         if self.mode == "index":
-            rc = self.lib.pmrl_rollout_gather_index(self.S, self.E, A, W, F, self.T, B, _lib.ptr(slots), _lib.ptr(envs),
+            gather_index = self.lib.pmrl_rollout_gather_index_bf16 if self._bf16 else self.lib.pmrl_rollout_gather_index
+            rc = gather_index(self.S, self.E, A, W, F, self.T, B, _lib.ptr(slots), _lib.ptr(envs),
                                                     _lib.ptr(self.bi), _lib.ptr(self.a), _lib.ptr(self.v), _lib.ptr(self.r),
                                                     _lib.ptr(self.wp), _lib.ptr(self.feat_am), _lib.ptr(self.y_tm),
                                                     _lib.ptr(s), _lib.ptr(a), _lib.ptr(r), _lib.ptr(pv), _lib.ptr(pa), _lib.ptr(p),
@@ -176,7 +194,8 @@ class DeviceRolloutBuffer:
             return s, a, r, pv, pa, p
         if self.s is None:
             raise _lib.PmrlError("this rollout buffer was built with store_obs=False")
-        rc = self.lib.pmrl_rollout_gather(self.S, self.E, A, W, F, B, _lib.ptr(slots), _lib.ptr(envs), _lib.ptr(self.s),
+        gather = self.lib.pmrl_rollout_gather_bf16 if self._bf16 else self.lib.pmrl_rollout_gather
+        rc = gather(self.S, self.E, A, W, F, B, _lib.ptr(slots), _lib.ptr(envs), _lib.ptr(self.s),
                                           _lib.ptr(self.a), _lib.ptr(self.v), _lib.ptr(self.r), _lib.ptr(self.y),
                                           _lib.ptr(s), _lib.ptr(a), _lib.ptr(r), _lib.ptr(pv), _lib.ptr(pa), _lib.ptr(p),
                                           _lib.current_stream())
@@ -210,11 +229,16 @@ class DeviceRolloutBuffer:
 
 
 class DeviceReplayBuffer:
+    """Off-policy index replay (replay/buffer.py:6-79, replay/traj_buffer.py:6-89).  obs_dtype="bfloat16": the windows
+    `gather` / `sample` regenerate (s, s_) are returned as bf16, rounded from the fp32 table and actions."""
+
     def __init__(self, feat_am, num_features: int, train_len: int, num_envs: int, num_assets: int, window_size: int,
-                 buffer_size: int = 425000, batch_size: int = 32, include_last: bool = True, device=None):
+                 buffer_size: int = 425000, batch_size: int = 32, include_last: bool = True, device=None,
+                 obs_dtype: str = "float32"):
         if not torch.cuda.is_available():
             raise _lib.PmrlError("DeviceReplayBuffer needs a CUDA device (pmrl_b200 has no CPU fallback)")
         self.lib = _lib.load()
+        self.obs_dtype = _obs_dtype(obs_dtype)
         self.feat_am = feat_am                                   # [A, T, F-1] device table (the `dataset`, buffer.py:8)
         self.T = feat_am.shape[1]
         self.F, self.E, self.A, self.W = num_features, num_envs, num_assets, window_size
@@ -284,9 +308,10 @@ class DeviceReplayBuffer:
         st = torch.as_tensor(starts).to(dev, torch.int32).contiguous()
         B = ep.numel()
         A, W, F = self.A, self.W, self.F
-        s = torch.empty(B, A, W, F, device=dev); s2 = torch.empty(B, A, W, F, device=dev)
+        s = torch.empty(B, A, W, F, dtype=self.obs_dtype, device=dev); s2 = torch.empty(B, A, W, F, dtype=self.obs_dtype, device=dev)
         a = torch.empty(B, A, 1, device=dev); r = torch.empty(B, 1, 1, device=dev)
-        rc = self.lib.pmrl_replay_gather(self.max_epoch, self.epoch_len, self.E, A, W, F, self.T, B, _lib.ptr(ep), _lib.ptr(en),
+        gather = self.lib.pmrl_replay_gather_bf16 if self.obs_dtype is torch.bfloat16 else self.lib.pmrl_replay_gather
+        rc = gather(self.max_epoch, self.epoch_len, self.E, A, W, F, self.T, B, _lib.ptr(ep), _lib.ptr(en),
                                          _lib.ptr(st), _lib.ptr(self.bi), _lib.ptr(self.ba), _lib.ptr(self.br),
                                          _lib.ptr(self.feat_am), _lib.ptr(s), _lib.ptr(a), _lib.ptr(r), _lib.ptr(s2),
                                          _lib.current_stream())

@@ -95,7 +95,8 @@ class TradingEnv:
         else:
             self.reward_name = cfg.reward if cfg.reward != "step_log" else "log_returns"
         # a single env, never "done" (the reference ends an episode at loader exhaustion), step reward = :99
-        self.cfg = EnvConfig(**{**cfg.__dict__, "num_envs": 1, "episode_len": 0, "reward": "step_log"})
+        # (fp32 obs whatever cfg.obs_dtype says: this shim mirrors the reference's fp32 `features` tensor)
+        self.cfg = EnvConfig(**{**cfg.__dict__, "num_envs": 1, "episode_len": 0, "reward": "step_log", "obs_dtype": "float32"})
         self._env = BatchedTradingEnv(self.cfg, prices=None, features=None, device=device)
         self.init_cash = self.cfg.initial_cash            # agent/dreamer/dreamer.py:197
         self.three_tuple = three_tuple

@@ -9,6 +9,7 @@ from __future__ import annotations
 from dataclasses import dataclass
 
 REWARD_MODES = {"step_log": 0, "returns": 1, "log_returns": 2, "sharpe_ratio": 3}
+OBS_DTYPES = ("float32", "bfloat16")
 
 
 @dataclass
@@ -25,6 +26,12 @@ class EnvConfig:
     episode_len: int = 1000           # steps per episode (the reference ends at loader exhaustion)
     mu_max_iter: int = 16             # cap for the commission fixed-point loop (trading_env.py:70)
     strict_reference: bool = True     # reproduce the AND-condition normalisation quirk (trading_env.py:58)
+    obs_dtype: str = "float32"        # "bfloat16": the kernels write the obs as bf16 (rounded from the fp32 values; state,
+                                      # rewards and everything else stay fp32) — half the obs bytes for a bf16 network
+
+    def __post_init__(self):
+        if self.obs_dtype not in OBS_DTYPES:
+            raise ValueError(f"unknown obs_dtype {self.obs_dtype!r}; expected one of {OBS_DTYPES}")
 
     @property
     def reward_mode(self) -> int:

@@ -171,8 +171,11 @@ __global__ void __launch_bounds__(kStepThreads) k_env_reset(const StepParams p) 
 // ------------------------------------------------------------------------------------------------
 // Observation tiles from the current state.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kObsThreads) k_obs_build(const StepParams p) {
-    extern __shared__ __align__(128) float tile[];
+// OT: obs element type (float, or uint16_t bf16 bits — PMRL_OBS_BF16); the fp32 and bf16 kernels below share this body.
+template <typename OT>
+__device__ __forceinline__ void obs_build(const StepParams& p) {
+    extern __shared__ __align__(128) unsigned char smem_obs[];
+    OT* const tile = reinterpret_cast<OT*>(smem_obs);
     const int e = blockIdx.x / p.tiles_per_env;
     const int ti = blockIdx.x - e * p.tiles_per_env;
     if (p.mask && !p.mask[e]) return;
@@ -190,6 +193,8 @@ __global__ void __launch_bounds__(kObsThreads) k_obs_build(const StepParams p) {
     obs_tile_store(p, tile, e, a0, na, tid, kObsThreads);
     if (p.obs_mode == PMRL_OBS_FULL && p.obs_bulk_ok && tid == 0) bulk_wait_read<0>();
 }
+__global__ void __launch_bounds__(kObsThreads) k_obs_build(const StepParams p) { obs_build<float>(p); }
+__global__ void __launch_bounds__(kObsThreads) k_obs_build_bf16(const StepParams p) { obs_build<uint16_t>(p); }
 
 
 // The same tile for the common shape (4 feature channels + weight slot, W <= 64, 32-asset tiles), without the
@@ -255,6 +260,70 @@ __global__ void __launch_bounds__(kObsThreads) k_obs_build_rows(const StepParams
     }
 }
 
+// k_obs_build_rows with the tile in obs element type OT (instantiated for bf16 bits: k_obs_build_rows_bf16).  The fp32
+// kernel above keeps its own code: compiled through this template its SASS comes out reordered.
+template <typename OT>
+__device__ __forceinline__ void obs_build_rows(const StepParams& p) {
+    extern __shared__ __align__(128) unsigned char smem_obs[];
+    OT* const tile = reinterpret_cast<OT*>(smem_obs);               // [32][W][5]
+    const int A = p.A, W = p.W, T = p.T;
+    const int e = blockIdx.x / p.tiles_per_env;
+    const int ti = blockIdx.x - e * p.tiles_per_env;
+    if (p.mask && !p.mask[e]) return;
+    const int a0 = ti * 32;
+    const int na = min(32, A - a0);
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int idx = p.idx[e], full = p.is_full[e];
+    const int row0 = p.t0[e] + p.t[e];
+    const int shift = full ? 0 : (W - idx);                         // weight_buffer.py:38-42
+    const bool w0 = lane < W, w1 = lane + 32 < W;
+    const float4* __restrict__ tbl = reinterpret_cast<const float4*>(p.feat_am) + ((size_t)a0 * T + row0 + lane);
+    float4 fv[4][2];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int al = warp + 8 * i;
+        if (al < na) {
+            const float4* __restrict__ src = tbl + (size_t)al * T;
+            if (w0) fv[i][0] = ld_keep4(src, kPolicyEvictLast);
+            if (w1) fv[i][1] = ld_keep4(src + 32, kPolicyEvictLast);
+        }
+    }
+    const float* __restrict__ ring = p.hist + (size_t)e * W * A + a0 + lane;
+    float rv[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const int w = warp + 8 * j, slot = w - shift;
+        rv[j] = (w < W && slot >= 0 && lane < na) ? ld_once(ring + (size_t)slot * A, kPolicyEvictFirst) : 0.0f;
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int al = warp + 8 * i;
+        if (al < na) {
+            OT* d = tile + (al * W + lane) * 5;
+            if (w0) { const float4 v = fv[i][0]; d[0] = obs_cvt<OT>(v.x); d[1] = obs_cvt<OT>(v.y); d[2] = obs_cvt<OT>(v.z); d[3] = obs_cvt<OT>(v.w); }
+            if (w1) { const float4 v = fv[i][1]; d[160] = obs_cvt<OT>(v.x); d[161] = obs_cvt<OT>(v.y); d[162] = obs_cvt<OT>(v.z); d[163] = obs_cvt<OT>(v.w); }
+        }
+    }
+    if (lane < na) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const int w = warp + 8 * j;
+            if (w < W) tile[(lane * W + w) * 5 + 4] = obs_cvt<OT>(rv[j]);
+        }
+    }
+    fence_proxy_async_smem();
+    __syncthreads();
+    OT* __restrict__ dst = reinterpret_cast<OT*>(p.obs) + ((size_t)e * A + a0) * W * 5;
+    const int n = na * W * 5;
+    if (((((uintptr_t)dst) | ((size_t)n * sizeof(OT))) & 15) == 0) {
+        if (tid == 0) { bulk_store_s2g(dst, tile, (uint32_t)n * (uint32_t)sizeof(OT), kPolicyEvictFirst); bulk_commit(); bulk_wait_read<0>(); }
+    } else {
+        for (int q = tid; q < n; q += kObsThreads) dst[q] = tile[q];
+    }
+}
+
+__global__ void __launch_bounds__(kObsThreads) k_obs_build_rows_bf16(const StepParams p) { obs_build_rows<uint16_t>(p); }
+
 }  // namespace pmrl
 
 // ================================================================================================
@@ -263,19 +332,19 @@ __global__ void __launch_bounds__(kObsThreads) k_obs_build_rows(const StepParams
 using namespace pmrl;
 
 // Pick the asset-tile of the obs kernels: the biggest tile ≤ cap bytes whose start offsets stay
-// 16-byte aligned (so the TMA bulk store applies) with the least ragged last tile.
-static void choose_obs_tile(int A, int W, int F, size_t cap_bytes, const void* obs, StepParams& p) {
-    const size_t per = (size_t)W * F * 4;
+// 16-byte aligned (so the TMA bulk store applies) with the least ragged last tile.  esz: bytes per obs element.
+static void choose_obs_tile(int A, int W, int F, size_t esz, size_t cap_bytes, const void* obs, StepParams& p) {
+    const size_t per = (size_t)W * F * esz;
     int max_ta = (int)(cap_bytes / per);
     if (max_ta > A) max_ta = A;
     if (max_ta < 1) max_ta = 1;
-    const bool env_aligned = (((size_t)A * W * F) % 4 == 0) && (((uintptr_t)obs) % 16 == 0);
+    const bool env_aligned = (((size_t)A * W * F * esz) % 16 == 0) && (((uintptr_t)obs) % 16 == 0);
     int best = -1; long best_waste = 0;
     if (env_aligned) {
         for (int pass = 0; pass < 2 && best < 0; ++pass) {
             const int lo = pass == 0 ? (max_ta + 1) / 2 : 1;
             for (int ta = max_ta; ta >= lo; --ta) {
-                if (((size_t)ta * W * F) % 4 != 0 && ta < A) continue;
+                if (((size_t)ta * W * F * esz) % 16 != 0 && ta < A) continue;
                 const long tiles = (A + ta - 1) / ta;
                 const long waste = tiles * ta - A;
                 if (best < 0 || waste < best_waste) { best = ta; best_waste = waste; }
@@ -308,9 +377,10 @@ static int fill_params(const PmrlEnvCfg* cfg, const PmrlTables* tbl, const PmrlE
     return 0;
 }
 
-static int check_obs_args(const StepParams& p, const float* obs, int obs_mode) {
-    if (obs_mode != PMRL_OBS_NONE && obs_mode != PMRL_OBS_FULL && obs_mode != PMRL_OBS_WEIGHTS)
-        return pmrl_fail(PMRL_E_ARG, "bad obs_mode");
+// obs_mode as passed by the caller (PMRL_OBS_BF16 included); the rest of the library works with the base mode and a bf16 flag
+static int check_obs_args(const StepParams& p, const float* obs, int obs_mode_arg) {
+    if (int rc = pmrl_check_obs_mode(obs_mode_arg)) return rc;
+    const int obs_mode = obs_mode_arg & ~PMRL_OBS_BF16;
     if (obs_mode == PMRL_OBS_NONE) return 0;
     if (!obs) return pmrl_fail(PMRL_E_ARG, "obs is NULL but obs_mode != NONE");
     if (p.F < 2 && obs_mode == PMRL_OBS_FULL) return pmrl_fail(PMRL_E_SHAPE, "F >= 2 required for a full obs");
@@ -329,22 +399,32 @@ static int check_obs_args(const StepParams& p, const float* obs, int obs_mode) {
 // Launch-shape knobs (pmrl_set_tuning).
 static int g_tune_group = 0, g_tune_ctas_per_sm = 0, g_tune_fused = 1, g_tune_fast = 1, g_tune_rt = 1;
 
-static int launch_obs(StepParams& p, float* obs, int obs_mode, cudaStream_t s) {
+// obs_mode: base mode (FULL / WEIGHTS); bf16: PMRL_OBS_BF16 was set (FULL only, checked by check_obs_args)
+static int launch_obs(StepParams& p, float* obs, int obs_mode, bool bf16, cudaStream_t s) {
     p.obs = obs; p.obs_mode = obs_mode;
+    const size_t esz = bf16 ? 2 : 4;
     if (obs_mode == PMRL_OBS_FULL && p.F == 5 && p.W <= 64 && p.t0 && g_tune_fast) {      // division-free tile kernel
         if (p.E == 0) return 0;
         p.tile_assets = 32;
         p.tiles_per_env = (p.A + 31) / 32;
         const long grid = (long)p.E * p.tiles_per_env;
         if (grid > 2147483647L) return pmrl_fail(PMRL_E_SHAPE, "E * tiles_per_env exceeds the grid limit");
+        if (bf16) {
+            k_obs_build_rows_bf16<<<(unsigned)grid, kObsThreads, (size_t)32 * p.W * 5 * esz, s>>>(p);
+            return pmrl_check_launch("k_obs_build_rows_bf16");
+        }
         k_obs_build_rows<<<(unsigned)grid, kObsThreads, (size_t)32 * p.W * 5 * 4, s>>>(p);
         return pmrl_check_launch("k_obs_build_rows");
     }
-    choose_obs_tile(p.A, p.W, p.F, kObsTileCapBytes, obs, p);
+    choose_obs_tile(p.A, p.W, p.F, esz, kObsTileCapBytes, obs, p);
     if (p.E == 0) return 0;
-    const size_t smem = (size_t)p.tile_assets * p.W * p.F * 4;
+    const size_t smem = (size_t)p.tile_assets * p.W * p.F * esz;
     const long grid = (long)p.E * p.tiles_per_env;
     if (grid > 2147483647L) return pmrl_fail(PMRL_E_SHAPE, "E * tiles_per_env exceeds the grid limit");
+    if (bf16) {
+        k_obs_build_bf16<<<(unsigned)grid, kObsThreads, smem, s>>>(p);
+        return pmrl_check_launch("k_obs_build_bf16");
+    }
     k_obs_build<<<(unsigned)grid, kObsThreads, smem, s>>>(p);
     return pmrl_check_launch("k_obs_build");
 }
@@ -430,14 +510,15 @@ extern "C" int pmrl_set_tuning(int32_t key, int32_t value) {
     }
 }
 
-static int launch_fused(StepParams& p, float* obs, int npl, int vec, cudaStream_t s) {
+static int launch_fused(StepParams& p, float* obs, int npl, int vec, bool bf16, cudaStream_t s) {
     p.obs = obs; p.obs_mode = PMRL_OBS_FULL;
     if (!g_tune_fast) return -100;
     if (g_tune_rt) {                                  // ring rows through one TMA bulk load per env (env_step_rt.cu)
         p.prefetch_next = (g_tune_rt == 2) ? 0 : 1;
-        const int rc = pmrl_launch_step_obs_rt(p, npl, vec, g_tune_group, g_tune_ctas_per_sm, s);
+        const int rc = pmrl_launch_step_obs_rt(p, npl, vec, g_tune_group, g_tune_ctas_per_sm, bf16, s);
         if (rc != -100) return rc;
     }
+    if (bf16) return -100;                            // no bf16 form of the register-staged kernel: its shapes take the two kernels
     // register-staged fill (env_step_fast.cu): F == 5, W <= 64, A <= 128 — the shapes RT's ring alignment excludes
     return pmrl_launch_step_obs_fast(p, npl, vec, g_tune_group, g_tune_ctas_per_sm, s);
     // -100: no fused kernel covers this shape (A > 128, F != 5, W > 64) → state-only step, then the obs tile kernel
@@ -455,7 +536,7 @@ extern "C" int pmrl_env_reset(const PmrlEnvCfg* cfg, const PmrlTables* tbl, cons
     const int cap = pmrl_sm_count() * 8;
     k_env_reset<<<want < cap ? want : cap, kStepThreads, 0, s>>>(p);
     if (int rc = pmrl_check_launch("k_env_reset")) return rc;
-    if (obs_mode != PMRL_OBS_NONE) return launch_obs(p, obs, obs_mode, s);
+    if (obs_mode != PMRL_OBS_NONE) return launch_obs(p, obs, obs_mode & ~PMRL_OBS_BF16, (obs_mode & PMRL_OBS_BF16) != 0, s);
     return 0;
 }
 
@@ -512,7 +593,7 @@ extern "C" int pmrl_obs_build(const PmrlEnvCfg* cfg, const PmrlTables* tbl, cons
     if (int rc = fill_params(cfg, tbl, st, p)) return rc;
     if (obs_mode == PMRL_OBS_NONE) return pmrl_fail(PMRL_E_ARG, "obs_mode NONE makes no obs");
     if (int rc = check_obs_args(p, obs, obs_mode)) return rc;
-    return launch_obs(p, obs, obs_mode, (cudaStream_t)stream);
+    return launch_obs(p, obs, obs_mode & ~PMRL_OBS_BF16, (obs_mode & PMRL_OBS_BF16) != 0, (cudaStream_t)stream);
 }
 
 // validation shared by the step entry points; fills the per-step fields of p
@@ -557,16 +638,17 @@ extern "C" int pmrl_env_step_io(const PmrlEnvCfg* cfg, const PmrlTables* tbl, co
     StepParams p;
     if (int rc = prepare_step(cfg, tbl, st, io, p)) return rc;
     float* obs = io->obs;
-    const int obs_mode = io->obs_mode;
-    if (int rc = check_obs_args(p, obs, obs_mode)) return rc;
+    if (int rc = check_obs_args(p, obs, io->obs_mode)) return rc;
+    const int obs_mode = io->obs_mode & ~PMRL_OBS_BF16;
+    const bool bf16 = (io->obs_mode & PMRL_OBS_BF16) != 0;
     const int npl = env_npl_for(p.A), vec = vec_for_pointers(p, npl);
     cudaStream_t s = (cudaStream_t)stream;
     if (obs_mode == PMRL_OBS_FULL && g_tune_fused && (size_t)p.W * p.F * 4 <= 36 * 1024) {
-        const int rc = launch_fused(p, obs, npl, vec, s);
+        const int rc = launch_fused(p, obs, npl, vec, bf16, s);
         if (rc != -100) return rc;                    // -100: no fused kernel for this shape → step kernel + obs kernel
     }
     if (int rc = launch_step_s(p, npl, vec, s)) return rc;
-    if (obs_mode != PMRL_OBS_NONE) return launch_obs(p, obs, obs_mode, s);
+    if (obs_mode != PMRL_OBS_NONE) return launch_obs(p, obs, obs_mode, bf16, s);
     return 0;
 }
 

@@ -118,9 +118,11 @@ extern "C" int pmrl_env_step_host(const PmrlEnvCfg* cfg, const PmrlTables* tbl, 
     if (!cfg || !tbl || !st || !actions_host || !actions_stage || !reward || !done || !reward_host || !done_host)
         return pmrl_fail(PMRL_E_ARG, "env_step_host: null argument");
     if (cfg->E <= 0 || cfg->A <= 0 || cfg->W <= 0 || cfg->F <= 0) return pmrl_fail(PMRL_E_SHAPE, "env_step_host: bad sizes");
+    if (int rc = pmrl_check_obs_mode(obs_mode)) return rc;
     if (obs_mode != PMRL_OBS_NONE && !obs) return pmrl_fail(PMRL_E_ARG, "env_step_host: obs_mode set but obs is null");
     cudaStream_t s = (cudaStream_t)stream;
-    const size_t A = (size_t)cfg->A, WA = (size_t)cfg->W * A, obs_env = WA * (size_t)cfg->F;
+    const size_t A = (size_t)cfg->A, WA = (size_t)cfg->W * A;
+    const size_t obs_env_bytes = WA * (size_t)cfg->F * ((obs_mode & PMRL_OBS_BF16) ? 2 : 4);   // bf16 obs: 2-byte elements
 
     if (slices == 0) {
         const float* act_dev = mapped_alias(actions_host);
@@ -133,7 +135,7 @@ extern "C" int pmrl_env_step_host(const PmrlEnvCfg* cfg, const PmrlTables* tbl, 
         // either way (131,072 x 100: 1.21 ms zero-copy vs 1.38 ms streamed; 262,144 x 500: 10.66 vs 9.94 ms); small batches lose
         // (4,096 x 50: 94 us vs 105 us).  No robust gain → zero-copy is the default and streaming stays an option.
         const size_t act_bytes = (size_t)cfg->E * A * sizeof(float);
-        const size_t stream_from = obs_mode == PMRL_OBS_FULL ? ((size_t)2 << 20) : ((size_t)128 << 20);
+        const size_t stream_from = (obs_mode & ~PMRL_OBS_BF16) == PMRL_OBS_FULL ? ((size_t)2 << 20) : ((size_t)128 << 20);
         if (act_dev && (g_host_stream == 2 || (g_host_stream == 1 && act_bytes >= stream_from))) {
             // streamed path (opt-in, PMRL_TUNE_HOST_STREAM): ONE kernel over the whole batch while the copy engine brings the action rows into
             // device memory chunk by chunk; every group of chunks is followed on the copy stream by its flag words, and
@@ -237,7 +239,7 @@ extern "C" int pmrl_env_step_host(const PmrlEnvCfg* cfg, const PmrlTables* tbl, 
         cst.sharpe = st->sharpe ? st->sharpe + 3 * (size_t)lo : nullptr;
         cst.ep_return = st->ep_return ? st->ep_return + lo : nullptr;
         int rc = pmrl_env_step(&ccfg, tbl, &cst, actions_stage + lo * A, nullptr, reward + lo, done + lo,
-                               obs ? obs + lo * obs_env : nullptr, obs_mode, stats, stream);
+                               obs ? (float*)((char*)obs + lo * obs_env_bytes) : nullptr, obs_mode, stats, stream);
         if (rc != 0) return drain(rc);
 
         PMRL_CUDA_DRAIN(cudaEventRecord(p->k_ev[c], s), "env_step_host: event record");

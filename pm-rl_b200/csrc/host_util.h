@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stddef.h>
+#include "pmrl_b200.h"
 
 // largest obs tile staged in shared memory by k_obs_build (fits the default 48 KB dynamic limit)
 static const size_t kObsTileCapBytes = 40 * 1024;
@@ -9,3 +10,11 @@ static const size_t kObsTileCapBytes = 40 * 1024;
 int pmrl_fail(int code, const char* msg);          // records msg for pmrl_last_error(), returns code
 int pmrl_check_launch(const char* what);           // cudaGetLastError() → 0 or positive cudaError_t
 int pmrl_sm_count(void);                           // SMs of the current device (cached per device)
+
+// obs_mode of the env entry points: PMRL_OBS_NONE / FULL / WEIGHTS, optionally | PMRL_OBS_BF16 with FULL.  0 or PMRL_E_ARG.
+static inline int pmrl_check_obs_mode(int obs_mode) {
+    const int base = obs_mode & ~PMRL_OBS_BF16;
+    if (base != PMRL_OBS_NONE && base != PMRL_OBS_FULL && base != PMRL_OBS_WEIGHTS) return pmrl_fail(PMRL_E_ARG, "bad obs_mode");
+    if ((obs_mode & PMRL_OBS_BF16) && base != PMRL_OBS_FULL) return pmrl_fail(PMRL_E_ARG, "bad obs_mode: PMRL_OBS_BF16 needs PMRL_OBS_FULL");
+    return 0;
+}

@@ -6,14 +6,16 @@
 //   get_all(): not full → zero front padding + chronological rows; full → raw ring order (quirk Q8)
 //                                           env/sim/weight_buffer.py:32-44
 // The tile is the exact byte image of the [na, W, F] slab of the reference obs layout, so it leaves
-// the SM as one contiguous TMA bulk store (cp.async.bulk shared::cta → global).
+// the SM as one contiguous TMA bulk store (cp.async.bulk shared::cta → global).  OT is the obs element type: float, or
+// uint16_t holding bf16 bits (PMRL_OBS_BF16: each element rounded from the fp32 value as the tile is filled).
 #pragma once
 #include "pmrl_device.cuh"
 
 namespace pmrl {
 
 // Feature channels 0..F-2 of the tile from the asset-major table (rows row0 .. row0+W-1).
-__device__ __forceinline__ void obs_tile_fill_features(const StepParams& p, float* __restrict__ tile,
+template <typename OT>
+__device__ __forceinline__ void obs_tile_fill_features(const StepParams& p, OT* __restrict__ tile,
                                                        int a0, int na, int row0, int tid, int nthreads) {
     const int W = p.W, F = p.F, Fm1 = p.F - 1, T = p.T;
     const uint64_t pol_keep = l2_policy_evict_last();
@@ -25,8 +27,8 @@ __device__ __forceinline__ void obs_tile_fill_features(const StepParams& p, floa
         for (int r = tid; r < n; r += nthreads) {
             const int al = r / W, w = r - al * W;
             const float4 v = ld_keep4(tbl + (size_t)(a0 + al) * T + row0 + w, pol_keep);
-            float* d = tile + r * 5;
-            d[0] = v.x; d[1] = v.y; d[2] = v.z; d[3] = v.w;
+            OT* d = tile + r * 5;
+            d[0] = obs_cvt<OT>(v.x); d[1] = obs_cvt<OT>(v.y); d[2] = obs_cvt<OT>(v.z); d[3] = obs_cvt<OT>(v.w);
         }
     } else {
         // any channel count: a warp owns an asset row of the tile (its window is ONE contiguous run of W·(F-1) floats in
@@ -38,10 +40,10 @@ __device__ __forceinline__ void obs_tile_fill_features(const StepParams& p, floa
         const int w_first = lane / Fm1, c_first = lane - w_first * Fm1;
         for (int al = warp; al < na; al += nwarps) {
             const float* __restrict__ src = p.feat_am + ((size_t)(a0 + al) * T + row0) * Fm1;
-            float* __restrict__ drow = tile + al * W * F;
+            OT* __restrict__ drow = tile + al * W * F;
             int w = w_first, c = c_first;
             for (int rem = lane; rem < per_asset; rem += 32) {
-                drow[w * F + c] = ld_keep(src + rem, pol_keep);
+                drow[w * F + c] = obs_cvt<OT>(ld_keep(src + rem, pol_keep));
                 w += dq; c += dr;
                 if (c >= Fm1) { c -= Fm1; ++w; }
             }
@@ -51,7 +53,8 @@ __device__ __forceinline__ void obs_tile_fill_features(const StepParams& p, floa
 
 // Weight channel F-1 of the tile from the ring (get_all semantics).  `fresh`/`fresh_slot`: optional
 // shared-memory copy of the row written by this very step (fused kernel), else fresh_slot = -1.
-__device__ __forceinline__ void obs_tile_fill_weights(const StepParams& p, float* __restrict__ tile,
+template <typename OT>
+__device__ __forceinline__ void obs_tile_fill_weights(const StepParams& p, OT* __restrict__ tile,
                                                       const float* __restrict__ hist_e, int a0, int na,
                                                       int idx, int is_full,
                                                       const float* __restrict__ fresh, int fresh_slot,
@@ -64,7 +67,7 @@ __device__ __forceinline__ void obs_tile_fill_weights(const StepParams& p, float
         for (int al = lane; al < na; al += 32) {
             float v = 0.0f;
             if (slot >= 0) v = (slot == fresh_slot) ? fresh[a0 + al] : ld_stream(hist_e + (size_t)slot * A + a0 + al);
-            tile[(al * W + w) * F + (F - 1)] = v;
+            tile[(al * W + w) * F + (F - 1)] = obs_cvt<OT>(v);
         }
     }
 }
@@ -72,16 +75,17 @@ __device__ __forceinline__ void obs_tile_fill_weights(const StepParams& p, float
 // Tile → obs.  mode FULL: whole slab (bulk store when aligned); mode WEIGHTS: channel F-1 only.
 // All threads of the CTA call this after `fence_proxy_async_smem(); __syncthreads();` following the
 // fills (every writer fences its own generic-proxy stores before the barrier, then one thread issues
-// the async-proxy bulk store).
-__device__ __forceinline__ void obs_tile_store(const StepParams& p, const float* __restrict__ tile,
+// the async-proxy bulk store).  WEIGHTS mode is fp32 only.
+template <typename OT>
+__device__ __forceinline__ void obs_tile_store(const StepParams& p, const OT* __restrict__ tile,
                                                int e, int a0, int na, int tid, int nthreads) {
     const int W = p.W, F = p.F;
-    float* __restrict__ dst = p.obs + ((size_t)e * p.A + a0) * W * F;
+    OT* __restrict__ dst = reinterpret_cast<OT*>(p.obs) + ((size_t)e * p.A + a0) * W * F;
     const int n = na * W * F;
     if (p.obs_mode == PMRL_OBS_FULL) {
         if (p.obs_bulk_ok) {
             if (tid == 0) {
-                bulk_store_s2g(dst, tile, (uint32_t)n * 4u, l2_policy_evict_first());
+                bulk_store_s2g(dst, tile, (uint32_t)n * (uint32_t)sizeof(OT), l2_policy_evict_first());
                 bulk_commit();
             }
         } else {

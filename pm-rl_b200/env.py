@@ -18,6 +18,8 @@ from . import _lib
 from .config import EnvConfig
 
 OBS_NONE, OBS_FULL, OBS_WEIGHTS = 0, 1, 2
+OBS_BF16 = 0x100                  # OR-ed into OBS_FULL: the obs is written as bf16 (include/pmrl_b200.h PMRL_OBS_BF16)
+OBS_TORCH_DTYPES = {"float32": torch.float32, "bfloat16": torch.bfloat16}
 STATS_LEN = 10
 STAT_NAMES = ("n_envs", "sum_r", "sum_r2", "sum_v", "sum_lnv", "n_done", "sum_ep_return", "sum_ep_len",
               "max_v", "max_neg_v")
@@ -39,6 +41,10 @@ class BatchedTradingEnv:
                    channel count is F-1); FFD'ed / scaled tables come from `pmrl_b200.features`.
         t0:        [E] int episode offsets into the table (default 0).
         collect_stats: accumulate the PMRL_STAT_* vector on device every step.
+
+    With `cfg.obs_dtype == "bfloat16"` every obs this env returns or writes (`reset`, `step`, `step_io`, `step_host`,
+    `graphed_step`, `observe`, and `out=` buffers, which must then be bfloat16) is the bf16 rounding of the fp32 obs;
+    state, rewards and the buffer rows written through `step_io` stay fp32.
     """
 
     @classmethod
@@ -56,6 +62,8 @@ class BatchedTradingEnv:
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
         E, A, W, F = cfg.num_envs, cfg.num_assets, cfg.window_size, cfg.num_features
         self.E, self.A, self.W, self.F = E, A, W, F
+        self.obs_dtype = OBS_TORCH_DTYPES[cfg.obs_dtype]
+        self._obs_full = OBS_FULL | (OBS_BF16 if self.obs_dtype is torch.bfloat16 else 0)   # obs_mode of every obs this env makes
         dev = self.device
         self.close_tm = None
         self.feat_am = None
@@ -154,11 +162,12 @@ class BatchedTradingEnv:
     # ------------------------------------------------------------------------------------------
     def _obs_buffer(self, out):
         if out is not None:
-            if out.shape != (self.E, self.A, self.W, self.F) or out.dtype != torch.float32:
-                raise ValueError(f"obs out must be float32 [{self.E}, {self.A}, {self.W}, {self.F}]")
+            if out.shape != (self.E, self.A, self.W, self.F) or out.dtype != self.obs_dtype:
+                raise ValueError(f"obs out must be {str(self.obs_dtype).replace('torch.', '')} [{self.E}, {self.A}, {self.W}, "
+                                 f"{self.F}] (the env's obs_dtype), got {out.dtype} {tuple(out.shape)}")
             return out
         if self._obs is None:
-            self._obs = torch.empty(self.E, self.A, self.W, self.F, dtype=torch.float32, device=self.device)
+            self._obs = torch.empty(self.E, self.A, self.W, self.F, dtype=self.obs_dtype, device=self.device)
         return self._obs
 
     def reset(self, mask=None, obs: bool = True, out=None):
@@ -170,7 +179,7 @@ class BatchedTradingEnv:
         want_obs = obs and self.feat_am is not None
         buf = self._obs_buffer(out) if want_obs else None
         rc = self.lib.pmrl_env_reset(self._p_cfg, self._p_tbl, self._p_st, _lib.ptr(m), _lib.ptr(buf),
-                                     OBS_FULL if want_obs else OBS_NONE, _lib.current_stream())
+                                     self._obs_full if want_obs else OBS_NONE, _lib.current_stream())
         _lib.check(rc, "pmrl_env_reset")
         return buf
 
@@ -191,7 +200,7 @@ class BatchedTradingEnv:
         buf = self._obs_buffer(out) if want_obs else None
         rc = self.lib.pmrl_env_step(self._p_cfg, self._p_tbl, self._p_st, a.data_ptr(), _lib.ptr(y),
                                     self._ptr_reward, self._ptr_done, buf.data_ptr() if buf is not None else None,
-                                    OBS_FULL if want_obs else OBS_NONE, self._ptr_stats,
+                                    self._obs_full if want_obs else OBS_NONE, self._ptr_stats,
                                     _lib.current_stream())
         if rc:
             _lib.check(rc, "pmrl_env_step")
@@ -221,7 +230,7 @@ class BatchedTradingEnv:
         io.actions, io.y_ext = a.data_ptr(), _lib.ptr(y)
         io.reward = reward.data_ptr() if reward is not None else self._ptr_reward
         io.done = done.data_ptr() if done is not None else self._ptr_done
-        io.obs, io.obs_mode, io.stats = _lib.ptr(buf), (OBS_FULL if want_obs else OBS_NONE), self._ptr_stats
+        io.obs, io.obs_mode, io.stats = _lib.ptr(buf), (self._obs_full if want_obs else OBS_NONE), self._ptr_stats
         io.action_sink, io.value_sink = _lib.ptr(action_sink), _lib.ptr(value_sink)
         io.weight_sink, io.index_sink = _lib.ptr(weight_sink), _lib.ptr(index_sink)
         io.reward_host = io.done_host = None
@@ -275,7 +284,7 @@ class BatchedTradingEnv:
         buf = self._obs_buffer(out) if want_obs else None
         rc = self.lib.pmrl_env_step_host(self._p_cfg, self._p_tbl, self._p_st, actions_host.data_ptr(), stage.data_ptr(),
                                          self.reward.data_ptr(), self.done.data_ptr(), reward_host.data_ptr(),
-                                         done_host.data_ptr(), _lib.ptr(buf), OBS_FULL if want_obs else OBS_NONE,
+                                         done_host.data_ptr(), _lib.ptr(buf), self._obs_full if want_obs else OBS_NONE,
                                          _lib.ptr(self._stats), int(chunks), _lib.current_stream())
         _lib.check(rc, "pmrl_env_step_host")
         return buf, reward_host, done_host
@@ -332,7 +341,9 @@ class BatchedTradingEnv:
         return static_actions, replay
 
     def write_weight_channel(self, obs):
-        """features[:, :, -1] = weights.get_all() on a caller-filled obs [E, A, W, F] (trading_env.py:103)."""
+        """features[:, :, -1] = weights.get_all() on a caller-filled obs [E, A, W, F] (trading_env.py:103).  fp32 envs only."""
+        if self.obs_dtype is not torch.float32:
+            raise _lib.PmrlError("write_weight_channel overwrites channel F-1 of a float32 obs; this env's obs_dtype is bfloat16")
         rc = self.lib.pmrl_obs_build(self._p_cfg, self._p_tbl, self._p_st, _lib.ptr(obs), OBS_WEIGHTS,
                                      _lib.current_stream())
         _lib.check(rc, "pmrl_obs_build")
@@ -341,7 +352,7 @@ class BatchedTradingEnv:
     def observe(self, out=None):
         """Materialise the obs of the current state without stepping."""
         buf = self._obs_buffer(out)
-        rc = self.lib.pmrl_obs_build(self._p_cfg, self._p_tbl, self._p_st, _lib.ptr(buf), OBS_FULL,
+        rc = self.lib.pmrl_obs_build(self._p_cfg, self._p_tbl, self._p_st, _lib.ptr(buf), self._obs_full,
                                      _lib.current_stream())
         _lib.check(rc, "pmrl_obs_build")
         return buf
