@@ -31,6 +31,7 @@
  *   pmrl_replay_gather  <- ReplayBuffer.sample           replay/buffer.py:39-79, replay/traj_buffer.py:45-89
  *   pmrl_pg_reward_*    <- PG._reward (fwd + grad wrt a) agent/pg/pg.py:40-82
  *   pmrl_eval_metrics   <- Metrics.sharpe/sortino/mdd/average_turnover  util/eval.py:14-37
+ *   pmrl_eval_stream_*  <- the same metrics, accumulated per step   util/eval.py:14-37
  *
  * Device data layout (all fp32 unless noted; E = envs on this GPU, A = assets incl.
  * cash at index 0, W = window, F = obs channels incl. the weight slot which is LAST):
@@ -395,6 +396,37 @@ int pmrl_pg_reward_fwd_bwd(int32_t B, int32_t A, int32_t mode, int32_t normalise
  *   turnover = mean_{i>=1} sum_a |w[i,a] - w[i-1,a]|                   (util/eval.py:32-37, pinned) */
 int pmrl_eval_metrics(const float* values, const float* weights, int32_t E, int32_t N, int32_t A,
                       float rf, int32_t periods, float* out, void* stream);
+
+/* Streaming form of the same metrics (util/eval.py:14-37): O(E) memory instead of [E, N] / [E, N, A] traces.
+ * acc is a caller-owned device buffer of E accumulators, PMRL_EVAL_ACC_BYTES each, 16-byte aligned; all-zero means
+ * "no episode seen".  Each holds the running episode (Welford mean / M2 of the excess returns, downside sum of squares,
+ * turnover sum in fp64; previous V, peak and min V/peak in fp32) and the record of completed episodes: the last one's
+ * (return, sharpe, sortino, mdd - 1, turnover), fp64 sums of those five and an episode count.
+ *
+ * pmrl_eval_stream_update: enqueue once after EVERY reset / step of the env batch (same stream).  Per env, with t the
+ * local step after the call: t == 0 restarts the running episode (V_prev = peak = V, the record is kept); t == last
+ * t + 1 adds the step (r = V/V_prev - 1 - ((1+rf)^(1/periods) - 1), turnover sum_a |w'_t - w'_{t-1}| from ring rows
+ * (idx-1) mod W and (idx-2) mod W) and, when t == episode_len (the step that returned done = 1), appends the episode to
+ * the record with its return ep_return[e]; t == last t does nothing; anything else (a missed update, or an accumulator
+ * that never saw a reset) marks the env invalid until its next reset.  rf / periods must be the same on every call.
+ * pmrl_eval_stream_read: out [E, 5] = (return, sharpe, sortino, mdd - 1, turnover) with the formulas of
+ * pmrl_eval_metrics (sd with ddof = 1, sortino over sqrt(downside / n), turnover = sum / n), for
+ *   which = PMRL_EVAL_RUNNING       the running episode (return = ep_return[e]); n = 0: sharpe, sortino, turnover NaN,
+ *                                    mdd 0; n = 1: sharpe NaN; an invalid env, or one stepped since its last update: NaN
+ *           PMRL_EVAL_LAST_EPISODE  the last completed episode (NaN without one)
+ *           PMRL_EVAL_EPISODE_MEAN  the mean of every completed episode's row (NaN without one)
+ * count [E] i32 (or NULL) receives the number of completed episodes.  rf is not used by the read (the update formed
+ * the excess returns); periods annualises sharpe and sortino.
+ * Both: NULL acc / value / hist / idx / t / ep_return (or out) → PMRL_E_ARG; E < 0, A outside [1, 1024], W < 2,
+ * periods < 1 → PMRL_E_SHAPE; acc not 16-byte aligned → PMRL_E_ALIGN; an unknown `which` → PMRL_E_ARG. */
+#define PMRL_EVAL_ACC_BYTES     128
+#define PMRL_EVAL_RUNNING       0
+#define PMRL_EVAL_LAST_EPISODE  1
+#define PMRL_EVAL_EPISODE_MEAN  2
+int pmrl_eval_stream_update(const PmrlEnvCfg* cfg, const PmrlEnvState* st, void* acc, float rf, int32_t periods,
+                            void* stream);
+int pmrl_eval_stream_read(const PmrlEnvCfg* cfg, const PmrlEnvState* st, const void* acc, int32_t which, float rf,
+                          int32_t periods, float* out, int32_t* count, void* stream);
 
 #ifdef __cplusplus
 }

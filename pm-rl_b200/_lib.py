@@ -89,7 +89,12 @@ SIGNATURES = {
     "pmrl_pg_reward_fwd_bwd": (C.c_int, [i32, i32, i32, i32, f32, f32, i32, c_void_p, c_void_p, c_void_p, c_void_p,
                                          c_void_p, c_void_p, f32, c_void_p]),
     "pmrl_eval_metrics": (C.c_int, [c_void_p, c_void_p, i32, i32, i32, f32, i32, c_void_p, c_void_p]),
+    "pmrl_eval_stream_update": (C.c_int, [P(PmrlEnvCfg), P(PmrlEnvState), c_void_p, f32, i32, c_void_p]),
+    "pmrl_eval_stream_read": (C.c_int, [P(PmrlEnvCfg), P(PmrlEnvState), c_void_p, i32, f32, i32, c_void_p, c_void_p,
+                                        c_void_p]),
 }
+
+EVAL_ACC_BYTES = 128       # include/pmrl_b200.h PMRL_EVAL_ACC_BYTES: one streaming-metrics accumulator per env
 
 _lib = None
 

@@ -82,7 +82,7 @@ extern "C" int pmrl_eval_metrics(const float* values, const float* weights, int3
     if (!values || !out) return pmrl_fail(PMRL_E_ARG, "eval_metrics: NULL pointer");
     if (E < 0 || N < 2 || A < 1 || periods < 1) return pmrl_fail(PMRL_E_SHAPE, "eval_metrics: need N >= 2, A >= 1, periods >= 1");
     if (E == 0) return 0;
-    const double rf_period = rf != 0.0f ? pow(1.0 + (double)rf, 1.0 / (double)periods) - 1.0 : 0.0;
+    const double rf_period = pmrl_rf_period(rf, periods);
     const int warps = kEvalThreads / 32;
     int blocks = (E + warps - 1) / warps;
     const int cap = pmrl_sm_count() * 8;

@@ -157,6 +157,7 @@ class BatchedTradingEnv:
         self._p_io = C.byref(self._io)
         self._p_cfg, self._p_tbl, self._p_st = C.byref(self._c_cfg), C.byref(self._c_tbl), C.byref(self._c_st)
         self._ptr_reward, self._ptr_done, self._ptr_stats = _lib.ptr(self.reward), _lib.ptr(self.done), _lib.ptr(self._stats)
+        self._eval = None                 # StreamingEvalMetrics fed after every reset / step (track_eval_metrics)
         self.reset(obs=False)
 
     # ------------------------------------------------------------------------------------------
@@ -181,6 +182,8 @@ class BatchedTradingEnv:
         rc = self.lib.pmrl_env_reset(self._p_cfg, self._p_tbl, self._p_st, _lib.ptr(m), _lib.ptr(buf),
                                      self._obs_full if want_obs else OBS_NONE, _lib.current_stream())
         _lib.check(rc, "pmrl_env_reset")
+        if self._eval is not None:
+            self._eval.update()
         return buf
 
     def step(self, actions, y=None, obs: bool = True, out=None):
@@ -204,6 +207,8 @@ class BatchedTradingEnv:
                                     _lib.current_stream())
         if rc:
             _lib.check(rc, "pmrl_env_step")
+        if self._eval is not None:
+            self._eval.update()
         return buf, self.reward, self.done
 
     def step_io(self, actions, y=None, obs: bool = True, out=None, reward=None, done=None, action_sink=None,
@@ -237,11 +242,16 @@ class BatchedTradingEnv:
         rc = self.lib.pmrl_env_step_io(self._p_cfg, self._p_tbl, self._p_st, self._p_io, _lib.current_stream())
         if rc:
             _lib.check(rc, "pmrl_env_step_io")
+        if self._eval is not None:
+            self._eval.update()
         return buf, (reward if reward is not None else self.reward), (done if done is not None else self.done)
 
     def step_burst(self, actions, reward=None, done=None):
         """K state-only steps in ONE launch on pre-supplied actions [K, E, A] (imagination bursts, HORIZON = 15 in
         config/dreamer.py:54): returns (reward [K, E], done [K, E]); bit-identical to K calls of `step(obs=False)`."""
+        if self._eval is not None:
+            raise _lib.PmrlError("step_burst: this env tracks evaluation metrics (track_eval_metrics), which need every "
+                                 "step's state; a burst keeps its intermediate states in registers — use step / graphed_step")
         a = actions
         if not (a.is_cuda and a.dtype is torch.float32 and a.is_contiguous() and a.dim() >= 2 and a[0].numel() == self.E * self.A):
             a = a.to(device=self.device, dtype=torch.float32).reshape(-1, self.E, self.A).contiguous()
@@ -287,6 +297,8 @@ class BatchedTradingEnv:
                                          done_host.data_ptr(), _lib.ptr(buf), self._obs_full if want_obs else OBS_NONE,
                                          _lib.ptr(self._stats), int(chunks), _lib.current_stream())
         _lib.check(rc, "pmrl_env_step_host")
+        if self._eval is not None:
+            self._eval.update()
         return buf, reward_host, done_host
 
     def graphed_step(self, obs: bool = True, out=None, steps: int = 1):
@@ -306,6 +318,8 @@ class BatchedTradingEnv:
         rew = torch.zeros(K, self.E, dtype=torch.float32, device=self.device) if K > 1 else None
         dn = torch.zeros(K, self.E, dtype=torch.uint8, device=self.device) if K > 1 else None
         state = (self.value, self.hist, self.idx, self.is_full, self.t, self.ep_return) + ((self.sharpe,) if self.sharpe is not None else ())
+        if self._eval is not None:
+            state += (self._eval.acc,)                    # the captured steps include the metrics update
 
         def burst():
             res = None
@@ -339,6 +353,19 @@ class BatchedTradingEnv:
             return result
 
         return static_actions, replay
+
+    def track_eval_metrics(self, rf: float = 0.0, periods: int = 252):
+        """Accumulate `loops.evaluate`'s metrics of every episode on the device as the env runs (util/eval.py:14-37),
+        in 128 bytes per env instead of value / weight traces.  From now on `reset`, `step`, `step_io`, `step_host` and
+        `graphed_step` (captured after this call) enqueue one `pmrl_eval_stream_update` right after their own launch;
+        `step_burst` raises.  Metrics start at each env's next reset: an env that is mid-episode now reads NaN until
+        then, an env at local step 0 starts at once.  A later call replaces the tracker.  Returns the
+        `metrics.StreamingEvalMetrics` (`running()`, `last_episode()`, `episode_mean()`, `clear()`)."""
+        from .metrics import StreamingEvalMetrics
+        tracker = StreamingEvalMetrics(self, rf=rf, periods=periods)
+        tracker.update()
+        self._eval = tracker
+        return tracker
 
     def write_weight_channel(self, obs):
         """features[:, :, -1] = weights.get_all() on a caller-filled obs [E, A, W, F] (trading_env.py:103).  fp32 envs only."""

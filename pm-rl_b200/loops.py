@@ -46,9 +46,30 @@ def collect_off_policy(env, act_fn, buffer, epoch: int, num_items: int):
 
 
 @torch.no_grad()
-def evaluate(env, act_fn, num_items: int, rf: float = 0.0, periods: int = 252):
-    """`Train._evaluate` (train/on_policy.py:76-90) batched: rolls one episode, keeps the value / weight traces on the
-    device and returns (total_reward [E], metrics [E, 4] = sharpe, sortino, max drawdown, average turnover)."""
+def evaluate(env, act_fn, num_items: int, rf: float = 0.0, periods: int = 252, traces: bool = True):
+    """`Train._evaluate` (train/on_policy.py:76-90) batched: rolls one episode and returns (total_reward [E],
+    metrics [E, 4] = sharpe, sortino, max drawdown, average turnover).
+
+    traces=True keeps the value / weight traces on the device ([E, N] + [E, N, A] floats) and computes the metrics from
+    them at the end.  traces=False feeds a `metrics.StreamingEvalMetrics` after every step instead (128 bytes per env):
+    the same total and drawdown bit for bit, Sharpe / Sortino / turnover up to the order of their fp64 sums.  It
+    evaluates exactly one episode, so it refuses num_items - 1 > env.cfg.episode_len."""
+    if not traces:
+        L = env.cfg.episode_len
+        if num_items < 2:
+            raise ValueError(f"evaluate: num_items must be >= 2 (one reset and at least one step), got {num_items}")
+        if L > 0 and num_items - 1 > L:
+            raise ValueError(f"evaluate(traces=False): {num_items - 1} steps cross the episode end "
+                             f"(episode_len = {L}); it evaluates exactly one episode")
+        from .metrics import StreamingEvalMetrics
+        tracker = StreamingEvalMetrics(env, rf=rf, periods=periods)
+        s = env.reset()
+        tracker.update()
+        for _ in range(1, num_items):
+            s, _, _ = env.step(act_fn(s))
+            tracker.update()
+        out, _ = tracker.running()
+        return out[:, 0].contiguous(), out[:, 1:].contiguous()
     from .metrics import eval_metrics
     s = env.reset()
     E, A = env.E, env.A
