@@ -32,6 +32,9 @@
  *   pmrl_pg_reward_*    <- PG._reward (fwd + grad wrt a) agent/pg/pg.py:40-82
  *   pmrl_eval_metrics   <- Metrics.sharpe/sortino/mdd/average_turnover  util/eval.py:14-37
  *   pmrl_eval_stream_*  <- the same metrics, accumulated per step   util/eval.py:14-37
+ *   pmrl_env_draw_starts<- the loader's episode start (every reset replays one fixed offset t0[e] otherwise);
+ *                          random starts as in online stochastic batch learning (Jiang, Xu & Liang 2017) and the
+ *                          recency-weighted sampling of replay/buffer.py (PERCENT_LATEST)
  *
  * Device data layout (all fp32 unless noted; E = envs on this GPU, A = assets incl.
  * cash at index 0, W = window, F = obs channels incl. the weight slot which is LAST):
@@ -170,7 +173,8 @@ typedef struct PmrlStepIO {
 #define PMRL_STAT_MAX_NEGV   9   /* max −V  (caller initialises to -inf) → min V = −this */
 
 int         pmrl_abi_version(void);
-/* sizeof of a boundary struct as compiled into the library (0 PmrlEnvCfg, 1 PmrlTables, 2 PmrlEnvState, 3 PmrlStepIO; 100+:
+/* sizeof of a boundary struct as compiled into the library (0 PmrlEnvCfg, 1 PmrlTables, 2 PmrlEnvState, 3 PmrlStepIO,
+ * 4 PmrlStartDist; 100+:
  * selected field offsets) — lets a foreign-language binding verify its mirror of the structs; -1 for an unknown code. */
 int         pmrl_abi_sizeof(int32_t which);
 const char* pmrl_last_error(void);
@@ -427,6 +431,48 @@ int pmrl_eval_stream_update(const PmrlEnvCfg* cfg, const PmrlEnvState* st, void*
                             void* stream);
 int pmrl_eval_stream_read(const PmrlEnvCfg* cfg, const PmrlEnvState* st, const void* acc, int32_t which, float rf,
                           int32_t periods, float* out, int32_t* count, void* stream);
+
+/* ---- randomised episode starts ---- */
+
+/* Draw a fresh table offset t0[e] for envs about to be reset, on the device (enqueue it BEFORE the reset / step call that
+ * reads the offset; the call after it then writes its obs, index_sink and every later row of the episode from the new t0).
+ *
+ * The draw of env e depends only on (seed, gid = env_base + e, episode[e]) — not on the stream, launch shape or how many
+ * GPUs share the batch:
+ *   (x0, x1, x2, x3) = Philox4x32-10(counter = (episode[e], gid & 0xffffffff, gid >> 32, 0),
+ *                                    key     = (seed & 0xffffffff, seed >> 32))          (Random123, Salmon et al. 2011)
+ *   r64 = (uint64)x0 << 32 | x1;   n = hi - lo + 1;   then episode[e] += 1 (u32)
+ *   PMRL_START_UNIFORM    t0 = lo + umul64hi(r64, n)                                      (integer only)
+ *   PMRL_START_GEOMETRIC  P(t0 = hi - j) ∝ beta (1 - beta)^j for j < n (recent rows favoured):
+ *                         u = (r64 >> 11) * 2^-53,  j = min(n - 1, floor(log1p(-u * geo_norm) / log1m_beta)),  t0 = hi - j
+ *                         with log1m_beta = log1p(-beta) and geo_norm = -expm1(n * log1m_beta), both double, from the caller
+ *                         (the device evaluates one fp64 log1p and one fp64 division per draw)
+ * mode PMRL_DRAW_DUE   draws for the envs the NEXT pmrl_env_step / _io / _host call auto-resets: episode_len > 0 and
+ *                      t[e] >= episode_len (the step kernels' own test); enqueue it right before that call.
+ *      PMRL_DRAW_MASK  draws for mask[e] != 0 (mask == NULL → every env); enqueue it right before pmrl_env_reset with the
+ *                      same mask.
+ * Envs that are not drawn are not written (t0 and episode keep their bytes).  t is read in DUE mode only (may be NULL
+ * otherwise).  t0 [E] i32 is the array PmrlEnvState.t0 points to, passed here writable; episode [E] u32 is caller-owned,
+ * zero-initialised for a fresh sequence.
+ * NULL cfg / dist / t0 / episode (or t in DUE mode), an unknown kind or mode, a geometric log1m_beta that is not finite
+ * and < 0 (beta outside (0, 1) or NaN) or a geo_norm outside (0, 1] → PMRL_E_ARG; E < 0, lo < 0, hi < lo, env_base outside
+ * [0, INT64_MAX - E] (global ids must not overflow),
+ * or T > 0 and hi + episode_len + W > T (the window of the last step would leave the tables) → PMRL_E_SHAPE. */
+#define PMRL_START_UNIFORM    0
+#define PMRL_START_GEOMETRIC  1
+#define PMRL_DRAW_DUE         0
+#define PMRL_DRAW_MASK        1
+typedef struct PmrlStartDist {
+    int32_t kind;              /* PMRL_START_* */
+    int32_t lo, hi;            /* offsets drawn from [lo, hi] */
+    int32_t pad;
+    uint64_t seed;             /* Philox key */
+    int64_t env_base;          /* global id of env 0 of this batch (a rank's first env) */
+    double log1m_beta;         /* GEOMETRIC: log1p(-beta) */
+    double geo_norm;           /* GEOMETRIC: -expm1((hi - lo + 1) * log1m_beta) */
+} PmrlStartDist;
+int pmrl_env_draw_starts(const PmrlEnvCfg* cfg, const PmrlStartDist* dist, const int32_t* t, const uint8_t* mask,
+                         int32_t mode, int32_t* t0, uint32_t* episode, void* stream);
 
 #ifdef __cplusplus
 }

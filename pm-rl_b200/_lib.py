@@ -39,6 +39,11 @@ class PmrlStepIO(C.Structure):
                 ("actions_ready", c_void_p), ("actions_ready_seq", C.c_uint32), ("actions_ready_shift", i32)]
 
 
+class PmrlStartDist(C.Structure):
+    _fields_ = [("kind", i32), ("lo", i32), ("hi", i32), ("pad", i32), ("seed", C.c_uint64), ("env_base", C.c_int64),
+                ("log1m_beta", C.c_double), ("geo_norm", C.c_double)]
+
+
 P = C.POINTER
 # symbol → (restype, argtypes); must list every function declared in include/pmrl_b200.h
 SIGNATURES = {
@@ -92,6 +97,8 @@ SIGNATURES = {
     "pmrl_eval_stream_update": (C.c_int, [P(PmrlEnvCfg), P(PmrlEnvState), c_void_p, f32, i32, c_void_p]),
     "pmrl_eval_stream_read": (C.c_int, [P(PmrlEnvCfg), P(PmrlEnvState), c_void_p, i32, f32, i32, c_void_p, c_void_p,
                                         c_void_p]),
+    "pmrl_env_draw_starts": (C.c_int, [P(PmrlEnvCfg), P(PmrlStartDist), c_void_p, c_void_p, i32, c_void_p, c_void_p,
+                                       c_void_p]),
 }
 
 EVAL_ACC_BYTES = 128       # include/pmrl_b200.h PMRL_EVAL_ACC_BYTES: one streaming-metrics accumulator per env

@@ -47,6 +47,7 @@ extern "C" int pmrl_abi_sizeof(int32_t which) {
         case 1: return (int)sizeof(PmrlTables);
         case 2: return (int)sizeof(PmrlEnvState);
         case 3: return (int)sizeof(PmrlStepIO);
+        case 4: return (int)sizeof(PmrlStartDist);
         case 100: return (int)offsetof(PmrlStepIO, stats);
         case 101: return (int)offsetof(PmrlStepIO, done_host);
         case 102: return (int)offsetof(PmrlEnvState, ticket);

@@ -225,7 +225,7 @@ __device__ __forceinline__ void env_load_scalars(const StepParams& p, int e, Env
 }
 
 __device__ __forceinline__ bool env_needs_reset(const StepParams& p, const EnvScalars& s) {
-    return p.episode_len > 0 && s.k >= p.episode_len;           // train/on_policy.py:60-61
+    return episode_due_reset(p.episode_len, s.k);                // train/on_policy.py:60-61
 }
 
 // Where the price relatives of the step after local step s.k live: the caller's [E, A] array or row t0 + k_new + W − 1 of the

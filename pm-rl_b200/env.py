@@ -39,7 +39,8 @@ class BatchedTradingEnv:
                    y_t = close_t / close_{t-1}, data/instrument.py:79), or None if every step gets `y=`.
         features:  [T, A, F-1] feature table gathered into the obs window (defaults to `prices` when its
                    channel count is F-1); FFD'ed / scaled tables come from `pmrl_b200.features`.
-        t0:        [E] int episode offsets into the table (default 0).
+        t0:        [E] int episode offsets into the table (default 0); redrawn at every reset once
+                   `sample_episode_starts` attaches a sampler.
         collect_stats: accumulate the PMRL_STAT_* vector on device every step.
 
     With `cfg.obs_dtype == "bfloat16"` every obs this env returns or writes (`reset`, `step`, `step_io`, `step_host`,
@@ -158,6 +159,7 @@ class BatchedTradingEnv:
         self._p_cfg, self._p_tbl, self._p_st = C.byref(self._c_cfg), C.byref(self._c_tbl), C.byref(self._c_st)
         self._ptr_reward, self._ptr_done, self._ptr_stats = _lib.ptr(self.reward), _lib.ptr(self.done), _lib.ptr(self._stats)
         self._eval = None                 # StreamingEvalMetrics fed after every reset / step (track_eval_metrics)
+        self._starts = None               # EpisodeStarts drawing t0 before every reset (sample_episode_starts)
         self.reset(obs=False)
 
     # ------------------------------------------------------------------------------------------
@@ -179,6 +181,8 @@ class BatchedTradingEnv:
             m = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
         want_obs = obs and self.feat_am is not None
         buf = self._obs_buffer(out) if want_obs else None
+        if self._starts is not None:
+            self._starts.draw_mask(m)
         rc = self.lib.pmrl_env_reset(self._p_cfg, self._p_tbl, self._p_st, _lib.ptr(m), _lib.ptr(buf),
                                      self._obs_full if want_obs else OBS_NONE, _lib.current_stream())
         _lib.check(rc, "pmrl_env_reset")
@@ -201,6 +205,8 @@ class BatchedTradingEnv:
             y = y.to(device=self.device, dtype=torch.float32).reshape(self.E, self.A).contiguous()
         want_obs = obs and self.feat_am is not None
         buf = self._obs_buffer(out) if want_obs else None
+        if self._starts is not None:
+            self._starts.draw_due()
         rc = self.lib.pmrl_env_step(self._p_cfg, self._p_tbl, self._p_st, a.data_ptr(), _lib.ptr(y),
                                     self._ptr_reward, self._ptr_done, buf.data_ptr() if buf is not None else None,
                                     self._obs_full if want_obs else OBS_NONE, self._ptr_stats,
@@ -239,6 +245,8 @@ class BatchedTradingEnv:
         io.action_sink, io.value_sink = _lib.ptr(action_sink), _lib.ptr(value_sink)
         io.weight_sink, io.index_sink = _lib.ptr(weight_sink), _lib.ptr(index_sink)
         io.reward_host = io.done_host = None
+        if self._starts is not None:
+            self._starts.draw_due()
         rc = self.lib.pmrl_env_step_io(self._p_cfg, self._p_tbl, self._p_st, self._p_io, _lib.current_stream())
         if rc:
             _lib.check(rc, "pmrl_env_step_io")
@@ -252,6 +260,9 @@ class BatchedTradingEnv:
         if self._eval is not None:
             raise _lib.PmrlError("step_burst: this env tracks evaluation metrics (track_eval_metrics), which need every "
                                  "step's state; a burst keeps its intermediate states in registers — use step / graphed_step")
+        if self._starts is not None:
+            raise _lib.PmrlError("step_burst: this env draws episode starts (sample_episode_starts); an episode ending inside "
+                                 "a burst would auto-reset with a stale t0 — use step / graphed_step, or detach() the sampler")
         a = actions
         if not (a.is_cuda and a.dtype is torch.float32 and a.is_contiguous() and a.dim() >= 2 and a[0].numel() == self.E * self.A):
             a = a.to(device=self.device, dtype=torch.float32).reshape(-1, self.E, self.A).contiguous()
@@ -292,6 +303,8 @@ class BatchedTradingEnv:
             stage = self._host_stage = torch.empty(E, A, dtype=torch.float32, device=self.device)
         want_obs = obs and self.feat_am is not None
         buf = self._obs_buffer(out) if want_obs else None
+        if self._starts is not None:
+            self._starts.draw_due()                       # every kernel of pmrl_env_step_host runs on this stream after it
         rc = self.lib.pmrl_env_step_host(self._p_cfg, self._p_tbl, self._p_st, actions_host.data_ptr(), stage.data_ptr(),
                                          self.reward.data_ptr(), self.done.data_ptr(), reward_host.data_ptr(),
                                          done_host.data_ptr(), _lib.ptr(buf), self._obs_full if want_obs else OBS_NONE,
@@ -320,6 +333,8 @@ class BatchedTradingEnv:
         state = (self.value, self.hist, self.idx, self.is_full, self.t, self.ep_return) + ((self.sharpe,) if self.sharpe is not None else ())
         if self._eval is not None:
             state += (self._eval.acc,)                    # the captured steps include the metrics update
+        if self._starts is not None:
+            state += (self.t0, self._starts.episodes)     # ... and the episode-start draws
 
         def burst():
             res = None
@@ -348,7 +363,9 @@ class BatchedTradingEnv:
         if stats_snap is not None:
             self._stats.copy_(stats_snap)
 
-        def replay():
+        # the graph holds raw pointers into `state` (the metrics accumulator and the sampler's draw counters among them):
+        # the closure keeps those tensors alive even if the tracker or sampler is replaced and dropped later
+        def replay(_keep=state):
             g.replay()
             return result
 
@@ -366,6 +383,27 @@ class BatchedTradingEnv:
         tracker.update()
         self._eval = tracker
         return tracker
+
+    def sample_episode_starts(self, low: int = 0, high=None, seed: int = 0, distribution: str = "uniform", beta=None,
+                              first_env: int = 0):
+        """Give every env a freshly drawn table offset t0[e] at each of its resets, on the device, instead of replaying the
+        offset it was built with.  From now on `reset(mask)` draws for the masked envs, and `step`, `step_io`, `step_host`
+        and `graphed_step` (captured after this call) draw for the envs the step auto-resets, each before its own launch;
+        `step_burst` raises.  The obs of a reset, `index_sink` and the rest of that episode use the new offset; between a
+        done step and the next call `t0` still holds the finished episode's start.  The first draw happens at each env's
+        next reset.
+
+        distribution "uniform" draws t0 uniformly from [low, high]; "geometric" draws t0 = high - j with
+        P(j) ∝ beta (1 - beta)^j, j < high - low + 1 (recent rows favoured).  high=None means T - episode_len - W.
+        first_env is the global id of env 0 (a rank passes `dist.shard_range(...)[0]`): a draw depends only on (seed,
+        global env id, that env's draw count).  A later call replaces the sampler.  Returns the `starts.EpisodeStarts`
+        (`episodes`: draws per env; `detach()`)."""
+        from .starts import EpisodeStarts, start_dist
+        dist = start_dist(self.T, self.cfg.episode_len, self.W, low=low, high=high, seed=seed, distribution=distribution,
+                          beta=beta, first_env=first_env)
+        sampler = EpisodeStarts(self, dist)
+        self._starts = sampler
+        return sampler
 
     def write_weight_channel(self, obs):
         """features[:, :, -1] = weights.get_all() on a caller-filled obs [E, A, W, F] (trading_env.py:103).  fp32 envs only."""
