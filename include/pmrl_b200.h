@@ -88,6 +88,27 @@ extern "C" {
                                    WEIGHTS | BF16, NONE | BF16 and unknown bits fail with PMRL_E_ARG before any launch.  A library
                                    built before this flag rejects it with "bad obs_mode" (PMRL_E_ARG): that is how a binding
                                    detects support (PMRL_ABI_VERSION is unchanged). */
+#define PMRL_OBS_REL     0x200  /* window-relative features (the price tensor of Jiang, Xu & Liang 2017): OR-ed into
+                                   PMRL_OBS_FULL, with or without PMRL_OBS_BF16, together with a reference channel `ref` (bits
+                                   10-13) and a channel mask (bits 14-29); build it with PMRL_OBS_REL_OF.  With r0 the first window
+                                   row the plain obs gathers for that env and call, the fp32 obs element is
+                                     obs[e, a, w, c]   = feat[r0 + w, a, c] / feat[r0 + W - 1, a, ref]   c in mask (IEEE fp32
+                                                                                                         division, __fdiv_rn bits)
+                                     obs[e, a, w, c]   = feat[r0 + w, a, c]                               c < F-1 not in mask
+                                     obs[e, a, w, F-1] = the weight channel, unchanged
+                                   and the bf16 obs (PMRL_OBS_BF16) is its round-to-nearest-even.  `ref` and every masked channel are
+                                   feature channels (< F-1).  A zero, denormal, negative, infinite or NaN divisor gives what IEEE
+                                   division gives (no check, no clamp); cash rows of 1 stay 1.  State, reward, done, stats, sinks
+                                   and everything else stay bit-identical to a plain FULL run.  Accepted by pmrl_env_reset,
+                                   pmrl_env_step, PmrlStepIO.obs_mode, pmrl_env_step_host, pmrl_obs_build and the two window-
+                                   regenerating gathers (pmrl_rollout_gather_index_obs, pmrl_replay_gather_obs).  NONE | REL,
+                                   WEIGHTS | REL, an empty mask, a mask bit or ref >= F-1 and unknown bits fail with PMRL_E_ARG,
+                                   F - 1 > 16 with REL fails with PMRL_E_SHAPE, both before any launch.  A library built before
+                                   this flag rejects it with "bad obs_mode" (PMRL_E_ARG). */
+#define PMRL_OBS_REL_REF_SHIFT  10
+#define PMRL_OBS_REL_MASK_SHIFT 14
+#define PMRL_OBS_REL_OF(ref, mask) \
+    (PMRL_OBS_REL | (((int32_t)(ref) & 0xF) << PMRL_OBS_REL_REF_SHIFT) | (((int32_t)(mask) & 0xFFFF) << PMRL_OBS_REL_MASK_SHIFT))
 
 typedef struct PmrlEnvCfg {
     int32_t E, A, W, F;        /* envs on this device, assets, window, obs channels (weight slot = F-1) */
@@ -378,6 +399,22 @@ int pmrl_replay_gather_bf16(int32_t P, int32_t L, int32_t E, int32_t A, int32_t 
                             const int32_t* epochs, const int32_t* envs, const int32_t* starts,
                             const int32_t* bi, const float* ba, const float* br, const float* feat_am,
                             uint16_t* s_out, float* a_out, float* r_out, uint16_t* s2_out, void* stream);
+
+/* The two window-regenerating gathers with the obs in any FULL form: obs_mode = PMRL_OBS_FULL, optionally | PMRL_OBS_BF16
+ * (s_out / s2_out hold bf16 bit patterns, else fp32), optionally | PMRL_OBS_REL_OF(ref, mask) (each regenerated window is
+ * divided like the env's: s by its own row i + W - 1 of feat_am, s' by row i + W), so that a sample equals the obs the env
+ * returned at that step.  Other parameters and outputs as pmrl_rollout_gather_index / pmrl_replay_gather; a bad obs_mode
+ * fails like it does for the env entry points. */
+int pmrl_rollout_gather_index_obs(int32_t S, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
+                                  const int32_t* slots, const int32_t* envs,
+                                  const int32_t* bi, const float* a, const float* v, const float* r,
+                                  const float* wp, const float* feat_am, const float* y_tm,
+                                  void* s_out, float* a_out, float* r_out, float* pv_out, float* pa_out, float* p_out,
+                                  int32_t obs_mode, void* stream);
+int pmrl_replay_gather_obs(int32_t P, int32_t L, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
+                           const int32_t* epochs, const int32_t* envs, const int32_t* starts,
+                           const int32_t* bi, const float* ba, const float* br, const float* feat_am,
+                           void* s_out, float* a_out, float* r_out, void* s2_out, int32_t obs_mode, void* stream);
 
 /* ---- differentiable batched reward (agent/pg/pg.py:40-82) ---- */
 

@@ -91,6 +91,12 @@ SIGNATURES = {
     "pmrl_replay_gather_bf16": (C.c_int, [i32, i32, i32, i32, i32, i32, i32, i32, c_void_p, c_void_p, c_void_p,
                                           c_void_p, c_void_p, c_void_p, c_void_p,
                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "pmrl_rollout_gather_index_obs": (C.c_int, [i32, i32, i32, i32, i32, i32, i32, c_void_p, c_void_p,
+                                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, i32, c_void_p]),
+    "pmrl_replay_gather_obs": (C.c_int, [i32, i32, i32, i32, i32, i32, i32, i32, c_void_p, c_void_p, c_void_p,
+                                         c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_void_p, c_void_p, c_void_p, c_void_p, i32, c_void_p]),
     "pmrl_pg_reward_fwd_bwd": (C.c_int, [i32, i32, i32, i32, f32, f32, i32, c_void_p, c_void_p, c_void_p, c_void_p,
                                          c_void_p, c_void_p, f32, c_void_p]),
     "pmrl_eval_metrics": (C.c_int, [c_void_p, c_void_p, i32, i32, i32, f32, i32, c_void_p, c_void_p]),

@@ -14,7 +14,9 @@ import numpy as np
 import torch
 
 from . import _lib
+from .config import obs_relative_bits, obs_relative_check
 
+_OBS_FULL, _OBS_BF16 = 1, 0x100                               # include/pmrl_b200.h PMRL_OBS_FULL, PMRL_OBS_BF16
 _OBS_DTYPES = {"float32": torch.float32, "bfloat16": torch.bfloat16}
 
 
@@ -41,11 +43,16 @@ class DeviceRolloutBuffer:
     the rows elsewhere.
 
     obs_dtype="bfloat16": s is stored (full mode) and returned by `gather` / `sample` / `sample_random` (both modes) as
-    bf16, half the bytes; the env feeding it must have the same obs_dtype.  a, v, r, prices stay fp32."""
+    bf16, half the bytes; the env feeding it must have the same obs_dtype.  a, v, r, prices stay fp32.
+
+    obs_relative_to / obs_relative_channels (index mode): the regenerated windows are window-relative like those of an env
+    with the same `EnvConfig` settings, so a sample equals the obs the env returned.  A full-mode buffer stores what the env
+    wrote and ignores them."""
 
     def __init__(self, num_features: int, train_len: int, num_envs: int, num_assets: int, window_size: int,
                  initial_cash: float = 25000.0, batch_size: int = 64, device=None, store_obs: bool = True,
-                 mode: str = "full", feat_am=None, y_tm=None, obs_dtype: str = "float32"):
+                 mode: str = "full", feat_am=None, y_tm=None, obs_dtype: str = "float32",
+                 obs_relative_to: int | None = None, obs_relative_channels=None):
         if not torch.cuda.is_available():
             raise _lib.PmrlError("DeviceRolloutBuffer needs a CUDA device (pmrl_b200 has no CPU fallback)")
         if mode not in ("full", "index"):
@@ -54,6 +61,9 @@ class DeviceRolloutBuffer:
         self.mode = mode
         self.obs_dtype = _obs_dtype(obs_dtype)
         self._bf16 = self.obs_dtype is torch.bfloat16
+        self.obs_relative_to = obs_relative_to
+        self.obs_relative_channels = obs_relative_check(obs_relative_to, obs_relative_channels, num_features)
+        self._obs_mode = _OBS_FULL | (_OBS_BF16 if self._bf16 else 0) | obs_relative_bits(obs_relative_to, self.obs_relative_channels)
         self.F, self.E, self.A, self.W = num_features, num_envs, num_assets, window_size
         self.step_offset = window_size - 1                      # rollout_buffer.py:10
         self.epoch_len = train_len - self.step_offset           # rollout_buffer.py:11
@@ -184,12 +194,11 @@ class DeviceRolloutBuffer:
         a = torch.empty(B, A, 1, device=dev); r = torch.empty(B, 1, 1, device=dev)
         pv = torch.empty(B, 1, 1, device=dev); pa = torch.empty(B, A, 1, device=dev); p = torch.empty(B, A, 1, device=dev)
         if self.mode == "index":
-            gather_index = self.lib.pmrl_rollout_gather_index_bf16 if self._bf16 else self.lib.pmrl_rollout_gather_index
-            rc = gather_index(self.S, self.E, A, W, F, self.T, B, _lib.ptr(slots), _lib.ptr(envs),
-                                                    _lib.ptr(self.bi), _lib.ptr(self.a), _lib.ptr(self.v), _lib.ptr(self.r),
-                                                    _lib.ptr(self.wp), _lib.ptr(self.feat_am), _lib.ptr(self.y_tm),
-                                                    _lib.ptr(s), _lib.ptr(a), _lib.ptr(r), _lib.ptr(pv), _lib.ptr(pa), _lib.ptr(p),
-                                                    _lib.current_stream())
+            rc = self.lib.pmrl_rollout_gather_index_obs(self.S, self.E, A, W, F, self.T, B, _lib.ptr(slots), _lib.ptr(envs),
+                                                        _lib.ptr(self.bi), _lib.ptr(self.a), _lib.ptr(self.v), _lib.ptr(self.r),
+                                                        _lib.ptr(self.wp), _lib.ptr(self.feat_am), _lib.ptr(self.y_tm),
+                                                        _lib.ptr(s), _lib.ptr(a), _lib.ptr(r), _lib.ptr(pv), _lib.ptr(pa),
+                                                        _lib.ptr(p), self._obs_mode, _lib.current_stream())
             _lib.check(rc, "pmrl_rollout_gather_index")
             return s, a, r, pv, pa, p
         if self.s is None:
@@ -230,15 +239,21 @@ class DeviceRolloutBuffer:
 
 class DeviceReplayBuffer:
     """Off-policy index replay (replay/buffer.py:6-79, replay/traj_buffer.py:6-89).  obs_dtype="bfloat16": the windows
-    `gather` / `sample` regenerate (s, s_) are returned as bf16, rounded from the fp32 table and actions."""
+    `gather` / `sample` regenerate (s, s_) are returned as bf16, rounded from the fp32 table and actions.
+    obs_relative_to / obs_relative_channels: s and s_ are window-relative like the obs of an env with the same `EnvConfig`
+    settings (each window divided by its own last row)."""
 
     def __init__(self, feat_am, num_features: int, train_len: int, num_envs: int, num_assets: int, window_size: int,
                  buffer_size: int = 425000, batch_size: int = 32, include_last: bool = True, device=None,
-                 obs_dtype: str = "float32"):
+                 obs_dtype: str = "float32", obs_relative_to: int | None = None, obs_relative_channels=None):
         if not torch.cuda.is_available():
             raise _lib.PmrlError("DeviceReplayBuffer needs a CUDA device (pmrl_b200 has no CPU fallback)")
         self.lib = _lib.load()
         self.obs_dtype = _obs_dtype(obs_dtype)
+        self.obs_relative_to = obs_relative_to
+        self.obs_relative_channels = obs_relative_check(obs_relative_to, obs_relative_channels, num_features)
+        self._obs_mode = (_OBS_FULL | (_OBS_BF16 if self.obs_dtype is torch.bfloat16 else 0)
+                          | obs_relative_bits(obs_relative_to, self.obs_relative_channels))
         self.feat_am = feat_am                                   # [A, T, F-1] device table (the `dataset`, buffer.py:8)
         self.T = feat_am.shape[1]
         self.F, self.E, self.A, self.W = num_features, num_envs, num_assets, window_size
@@ -310,11 +325,10 @@ class DeviceReplayBuffer:
         A, W, F = self.A, self.W, self.F
         s = torch.empty(B, A, W, F, dtype=self.obs_dtype, device=dev); s2 = torch.empty(B, A, W, F, dtype=self.obs_dtype, device=dev)
         a = torch.empty(B, A, 1, device=dev); r = torch.empty(B, 1, 1, device=dev)
-        gather = self.lib.pmrl_replay_gather_bf16 if self.obs_dtype is torch.bfloat16 else self.lib.pmrl_replay_gather
-        rc = gather(self.max_epoch, self.epoch_len, self.E, A, W, F, self.T, B, _lib.ptr(ep), _lib.ptr(en),
-                                         _lib.ptr(st), _lib.ptr(self.bi), _lib.ptr(self.ba), _lib.ptr(self.br),
-                                         _lib.ptr(self.feat_am), _lib.ptr(s), _lib.ptr(a), _lib.ptr(r), _lib.ptr(s2),
-                                         _lib.current_stream())
+        rc = self.lib.pmrl_replay_gather_obs(self.max_epoch, self.epoch_len, self.E, A, W, F, self.T, B, _lib.ptr(ep),
+                                             _lib.ptr(en), _lib.ptr(st), _lib.ptr(self.bi), _lib.ptr(self.ba), _lib.ptr(self.br),
+                                             _lib.ptr(self.feat_am), _lib.ptr(s), _lib.ptr(a), _lib.ptr(r), _lib.ptr(s2),
+                                             self._obs_mode, _lib.current_stream())
         _lib.check(rc, "pmrl_replay_gather")
         return s, a, r, s2
 

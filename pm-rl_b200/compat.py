@@ -95,8 +95,9 @@ class TradingEnv:
         else:
             self.reward_name = cfg.reward if cfg.reward != "step_log" else "log_returns"
         # a single env, never "done" (the reference ends an episode at loader exhaustion), step reward = :99
-        # (fp32 obs whatever cfg.obs_dtype says: this shim mirrors the reference's fp32 `features` tensor)
-        self.cfg = EnvConfig(**{**cfg.__dict__, "num_envs": 1, "episode_len": 0, "reward": "step_log", "obs_dtype": "float32"})
+        # (plain fp32 obs whatever cfg.obs_dtype / obs_relative_to say: this shim mirrors the reference's fp32 `features` tensor)
+        self.cfg = EnvConfig(**{**cfg.__dict__, "num_envs": 1, "episode_len": 0, "reward": "step_log", "obs_dtype": "float32",
+                                          "obs_relative_to": None, "obs_relative_channels": None})
         self._env = BatchedTradingEnv(self.cfg, prices=None, features=None, device=device)
         self.init_cash = self.cfg.initial_cash            # agent/dreamer/dreamer.py:197
         self.three_tuple = three_tuple

@@ -8,6 +8,7 @@ from __future__ import annotations
 
 from dataclasses import dataclass
 
+OBS_REL, OBS_REL_REF_SHIFT, OBS_REL_MASK_SHIFT = 0x200, 10, 14   # include/pmrl_b200.h PMRL_OBS_REL, PMRL_OBS_REL_OF
 REWARD_MODES = {"step_log": 0, "returns": 1, "log_returns": 2, "sharpe_ratio": 3}
 OBS_DTYPES = ("float32", "bfloat16")
 
@@ -28,10 +29,19 @@ class EnvConfig:
     strict_reference: bool = True     # reproduce the AND-condition normalisation quirk (trading_env.py:58)
     obs_dtype: str = "float32"        # "bfloat16": the kernels write the obs as bf16 (rounded from the fp32 values; state,
                                       # rewards and everything else stay fp32) — half the obs bytes for a bf16 network
+    obs_relative_to: int | None = None   # window-relative obs (Jiang, Xu & Liang 2017): the channels of every asset's window
+                                      # divided by this feature channel of its latest row (e.g. 3 = close); None = raw values
+    obs_relative_channels: tuple[int, ...] | None = None   # the feature channels divided (default: all, 0 .. F-2)
 
     def __post_init__(self):
         if self.obs_dtype not in OBS_DTYPES:
             raise ValueError(f"unknown obs_dtype {self.obs_dtype!r}; expected one of {OBS_DTYPES}")
+        self.obs_relative_channels = obs_relative_check(self.obs_relative_to, self.obs_relative_channels, self.num_features)
+
+    @property
+    def obs_relative_bits(self) -> int:
+        """The PMRL_OBS_REL bits of obs_mode for this config (0 when the obs is not window-relative)."""
+        return obs_relative_bits(self.obs_relative_to, self.obs_relative_channels)
 
     @property
     def reward_mode(self) -> int:
@@ -49,3 +59,34 @@ class EnvConfig:
                   risk_free_rate=float(cb.RISK_FREE_RATE))
         kw.update(overrides)
         return cls(**kw)
+
+
+def obs_relative_check(ref, channels, num_features: int):
+    """Validate a window-relative obs setting against F = num_features; returns the channels as a sorted tuple (every feature
+    channel 0 .. F-2 when `channels` is None), or None when `ref` is None."""
+    if ref is None:
+        if channels is not None:
+            raise ValueError("obs_relative_channels needs obs_relative_to (the divisor channel)")
+        return None
+    n = num_features - 1
+    if n > 16:
+        raise ValueError(f"window-relative obs covers at most 16 feature channels; num_features = {num_features}")
+    if isinstance(ref, bool) or not isinstance(ref, int) or not 0 <= ref < n:
+        raise ValueError(f"obs_relative_to must be a feature channel in [0, {n}), got {ref!r}")
+    chans = tuple(range(n)) if channels is None else tuple(channels)
+    if not chans:
+        raise ValueError("obs_relative_channels must name at least one channel")
+    for c in chans:
+        if isinstance(c, bool) or not isinstance(c, int) or not 0 <= c < n:
+            raise ValueError(f"obs_relative_channels must be feature channels in [0, {n}), got {c!r}")
+    return tuple(sorted(set(chans)))
+
+
+def obs_relative_bits(ref, channels) -> int:
+    """PMRL_OBS_REL_OF(ref, mask) for validated (ref, channels); 0 when ref is None."""
+    if ref is None:
+        return 0
+    mask = 0
+    for c in channels:
+        mask |= 1 << c
+    return OBS_REL | (ref << OBS_REL_REF_SHIFT) | (mask << OBS_REL_MASK_SHIFT)

@@ -163,10 +163,11 @@ __global__ void __launch_bounds__(kCopyThreads) k_replay_gather(const ReplayGath
     }
     if (p.obs_bulk_ok && tid == 0) bulk_wait_read<0>();
 }
-// k_replay_gather with the obs in element type OT (instantiated for bf16 bits: k_replay_gather_bf16; the fp32 kernel above keeps
-// its own code, whose SASS the template would reorder).
-template <typename OT>
-__device__ __forceinline__ void replay_gather(const ReplayGatherParams& g) {
+// k_replay_gather with the obs in element type OT (instantiated for bf16 bits: k_replay_gather_bf16, and with REL — window-relative
+// features, PMRL_OBS_REL — for both types: k_replay_gather_rel; the fp32 kernel above keeps its own code, whose SASS the template
+// would reorder).
+template <typename OT, bool REL = false>
+__device__ __forceinline__ void replay_gather(const ReplayGatherParams& g, const ObsRel& rel = ObsRel{0, 0u}) {
     extern __shared__ __align__(128) unsigned char smem_tile[];
     OT* const tile = reinterpret_cast<OT*>(smem_tile);
     StepParams p = g.p;
@@ -179,7 +180,7 @@ __device__ __forceinline__ void replay_gather(const ReplayGatherParams& g) {
     const int i = g.bi[(le + end - 1) * g.E + env];                   // stored loader index (buffer.py:65)
     const int a0 = ti * p.tile_assets;
     const int na = min(p.tile_assets, A - a0);
-    obs_tile_fill_features(p, tile, a0, na, i + which, tid, kCopyThreads);
+    obs_tile_fill_features<OT, REL>(p, tile, a0, na, i + which, tid, kCopyThreads, rel);
     // channel F-1 ← a_hist[:, which : which+W]ᵀ  (buffer.py:69-70); asset fastest → coalesced action rows
     const int n = W * na;
     for (int q = tid; q < n; q += kCopyThreads) {
@@ -199,6 +200,10 @@ __device__ __forceinline__ void replay_gather(const ReplayGatherParams& g) {
     if (p.obs_bulk_ok && tid == 0) bulk_wait_read<0>();
 }
 __global__ void __launch_bounds__(kCopyThreads) k_replay_gather_bf16(const ReplayGatherParams g) { replay_gather<uint16_t>(g); }
+template <typename OT>
+__global__ void __launch_bounds__(kCopyThreads) k_replay_gather_rel(const ReplayGatherParams g, const ObsRel rel) {
+    replay_gather<OT, true>(g, rel);
+}
 
 // Index-mode rollout gather: the buffer keeps (loader index, raw action, value, reward) per slot plus the un-wrapped history of
 // post-drift weights, and the observation s[slot] is REGENERATED here — feature window by index from the device table, weight
@@ -252,10 +257,10 @@ __global__ void __launch_bounds__(kCopyThreads) k_rollout_gather_index(const Rol
     }
     if (p.obs_bulk_ok && tid == 0) bulk_wait_read<0>();
 }
-// k_rollout_gather_index with the obs in element type OT (instantiated for bf16 bits: k_rollout_gather_index_bf16; the fp32 kernel above keeps
-// its own code, whose SASS the template would reorder).
-template <typename OT>
-__device__ __forceinline__ void rollout_gather_index(const RolloutIndexGatherParams& g) {
+// k_rollout_gather_index with the obs in element type OT (instantiated for bf16 bits: k_rollout_gather_index_bf16, and with REL for
+// both types: k_rollout_gather_index_rel; the fp32 kernel above keeps its own code, whose SASS the template would reorder).
+template <typename OT, bool REL = false>
+__device__ __forceinline__ void rollout_gather_index(const RolloutIndexGatherParams& g, const ObsRel& rel = ObsRel{0, 0u}) {
     extern __shared__ __align__(128) unsigned char smem_tile[];
     OT* const tile = reinterpret_cast<OT*>(smem_tile);
     StepParams p = g.p;
@@ -268,7 +273,7 @@ __device__ __forceinline__ void rollout_gather_index(const RolloutIndexGatherPar
     const int t = slot + g.off - 1;                                   // steps taken when that obs was made (>= W - 1: ring full)
     const int a0 = ti * p.tile_assets;
     const int na = min(p.tile_assets, A - a0);
-    obs_tile_fill_features(p, tile, a0, na, i - 1, tid, kCopyThreads);
+    obs_tile_fill_features<OT, REL>(p, tile, a0, na, i - 1, tid, kCopyThreads, rel);
     const int n = W * na;
     for (int q = tid; q < n; q += kCopyThreads) {
         const int w = q / na, al = q - w * na;                        // asset fastest → coalesced history rows
@@ -295,6 +300,10 @@ __device__ __forceinline__ void rollout_gather_index(const RolloutIndexGatherPar
 }
 __global__ void __launch_bounds__(kCopyThreads) k_rollout_gather_index_bf16(const RolloutIndexGatherParams g) {
     rollout_gather_index<uint16_t>(g);
+}
+template <typename OT>
+__global__ void __launch_bounds__(kCopyThreads) k_rollout_gather_index_rel(const RolloutIndexGatherParams g, const ObsRel rel) {
+    rollout_gather_index<OT, true>(g, rel);
 }
 
 }  // namespace pmrl
@@ -402,11 +411,11 @@ static void choose_tile(int A, int W, int F, size_t esz, const void* o1, const v
     p.tiles_per_env = (A + p.tile_assets - 1) / p.tile_assets;
 }
 
-// s_out / s2_out: float, or uint16_t bf16 bits (bf16 = true)
+// s_out / s2_out: float, or uint16_t bf16 bits (bf16 = true); rel: window-relative features (mask 0: off)
 static int replay_gather(int32_t P, int32_t L, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
                          const int32_t* epochs, const int32_t* envs, const int32_t* starts,
                          const int32_t* bi, const float* ba, const float* br, const float* feat_am,
-                         void* s_out, float* a_out, float* r_out, void* s2_out, bool bf16, void* stream) {
+                         void* s_out, float* a_out, float* r_out, void* s2_out, bool bf16, const ObsRel& rel, void* stream) {
     if (P < 1 || L < 1 || E < 1 || A < 1 || W < 1 || F < 2 || T < W + 1 || B < 0) return pmrl_fail(PMRL_E_SHAPE, "replay_gather: bad sizes");
     if (!epochs || !envs || !starts || !bi || !ba || !br || !feat_am || !s_out || !a_out || !r_out || !s2_out)
         return pmrl_fail(PMRL_E_ARG, "replay_gather: NULL pointer");
@@ -422,6 +431,11 @@ static int replay_gather(int32_t P, int32_t L, int32_t E, int32_t A, int32_t W, 
     g.epochs = epochs; g.envs = envs; g.starts = starts; g.bi = bi; g.ba = ba; g.br = br;
     g.s_out = (float*)s_out; g.a_out = a_out; g.r_out = r_out; g.s2_out = (float*)s2_out;
     const size_t smem = (size_t)g.p.tile_assets * W * F * esz;
+    if (rel.mask) {
+        if (bf16) k_replay_gather_rel<uint16_t><<<dim3(B, g.p.tiles_per_env, 2), kCopyThreads, smem, (cudaStream_t)stream>>>(g, rel);
+        else k_replay_gather_rel<float><<<dim3(B, g.p.tiles_per_env, 2), kCopyThreads, smem, (cudaStream_t)stream>>>(g, rel);
+        return pmrl_check_launch(bf16 ? "k_replay_gather_rel<bf16>" : "k_replay_gather_rel<float>");
+    }
     if (bf16) {
         k_replay_gather_bf16<<<dim3(B, g.p.tiles_per_env, 2), kCopyThreads, smem, (cudaStream_t)stream>>>(g);
         return pmrl_check_launch("k_replay_gather_bf16");
@@ -434,23 +448,23 @@ extern "C" int pmrl_replay_gather(int32_t P, int32_t L, int32_t E, int32_t A, in
                                   const int32_t* epochs, const int32_t* envs, const int32_t* starts,
                                   const int32_t* bi, const float* ba, const float* br, const float* feat_am,
                                   float* s_out, float* a_out, float* r_out, float* s2_out, void* stream) {
-    return replay_gather(P, L, E, A, W, F, T, B, epochs, envs, starts, bi, ba, br, feat_am, s_out, a_out, r_out, s2_out, false, stream);
+    return replay_gather(P, L, E, A, W, F, T, B, epochs, envs, starts, bi, ba, br, feat_am, s_out, a_out, r_out, s2_out, false, ObsRel{0, 0u}, stream);
 }
 
 extern "C" int pmrl_replay_gather_bf16(int32_t P, int32_t L, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
                                        const int32_t* epochs, const int32_t* envs, const int32_t* starts,
                                        const int32_t* bi, const float* ba, const float* br, const float* feat_am,
                                        uint16_t* s_out, float* a_out, float* r_out, uint16_t* s2_out, void* stream) {
-    return replay_gather(P, L, E, A, W, F, T, B, epochs, envs, starts, bi, ba, br, feat_am, s_out, a_out, r_out, s2_out, true, stream);
+    return replay_gather(P, L, E, A, W, F, T, B, epochs, envs, starts, bi, ba, br, feat_am, s_out, a_out, r_out, s2_out, true, ObsRel{0, 0u}, stream);
 }
 
-// s_out: float, or uint16_t bf16 bits (bf16 = true)
+// s_out: float, or uint16_t bf16 bits (bf16 = true); rel: window-relative features (mask 0: off)
 static int rollout_gather_index(int32_t S, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
                                 const int32_t* slots, const int32_t* envs,
                                 const int32_t* bi, const float* a, const float* v, const float* r,
                                 const float* wp, const float* feat_am, const float* y_tm,
                                 void* s_out, float* a_out, float* r_out, float* pv_out, float* pa_out, float* p_out,
-                                bool bf16, void* stream) {
+                                bool bf16, const ObsRel& rel, void* stream) {
     if (S < 2 || E < 1 || A < 1 || W < 2 || F < 2 || T < W + 1 || B < 0) return pmrl_fail(PMRL_E_SHAPE, "rollout_gather_index: bad sizes");
     if (!slots || !envs || !bi || !a || !v || !r || !wp || !feat_am || !y_tm || !s_out || !a_out || !r_out || !pv_out || !pa_out || !p_out)
         return pmrl_fail(PMRL_E_ARG, "rollout_gather_index: NULL pointer");
@@ -466,6 +480,11 @@ static int rollout_gather_index(int32_t S, int32_t E, int32_t A, int32_t W, int3
     g.slots = slots; g.envs = envs; g.bi = bi; g.a = a; g.v = v; g.r = r; g.wp = wp; g.y_tm = y_tm;
     g.s_out = (float*)s_out; g.a_out = a_out; g.r_out = r_out; g.pv_out = pv_out; g.pa_out = pa_out; g.p_out = p_out;
     const size_t smem = (size_t)g.p.tile_assets * W * F * esz;
+    if (rel.mask) {
+        if (bf16) k_rollout_gather_index_rel<uint16_t><<<dim3(B, g.p.tiles_per_env), kCopyThreads, smem, (cudaStream_t)stream>>>(g, rel);
+        else k_rollout_gather_index_rel<float><<<dim3(B, g.p.tiles_per_env), kCopyThreads, smem, (cudaStream_t)stream>>>(g, rel);
+        return pmrl_check_launch(bf16 ? "k_rollout_gather_index_rel<bf16>" : "k_rollout_gather_index_rel<float>");
+    }
     if (bf16) {
         k_rollout_gather_index_bf16<<<dim3(B, g.p.tiles_per_env), kCopyThreads, smem, (cudaStream_t)stream>>>(g);
         return pmrl_check_launch("k_rollout_gather_index_bf16");
@@ -481,7 +500,7 @@ extern "C" int pmrl_rollout_gather_index(int32_t S, int32_t E, int32_t A, int32_
                                          float* s_out, float* a_out, float* r_out, float* pv_out, float* pa_out, float* p_out,
                                          void* stream) {
     return rollout_gather_index(S, E, A, W, F, T, B, slots, envs, bi, a, v, r, wp, feat_am, y_tm, s_out, a_out, r_out, pv_out,
-                                pa_out, p_out, false, stream);
+                                pa_out, p_out, false, ObsRel{0, 0u}, stream);
 }
 
 extern "C" int pmrl_rollout_gather_index_bf16(int32_t S, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
@@ -491,5 +510,32 @@ extern "C" int pmrl_rollout_gather_index_bf16(int32_t S, int32_t E, int32_t A, i
                                               uint16_t* s_out, float* a_out, float* r_out, float* pv_out, float* pa_out,
                                               float* p_out, void* stream) {
     return rollout_gather_index(S, E, A, W, F, T, B, slots, envs, bi, a, v, r, wp, feat_am, y_tm, s_out, a_out, r_out, pv_out,
-                                pa_out, p_out, true, stream);
+                                pa_out, p_out, true, ObsRel{0, 0u}, stream);
+}
+
+// obs_mode of the two gathers below: PMRL_OBS_FULL, optionally | PMRL_OBS_BF16 and | PMRL_OBS_REL_OF(ref, mask)
+static int check_gather_obs_mode(int32_t obs_mode, int32_t F) {
+    if (int rc = pmrl_check_obs_mode(obs_mode, F)) return rc;
+    if ((obs_mode & 0xFF) != PMRL_OBS_FULL) return pmrl_fail(PMRL_E_ARG, "bad obs_mode: the gathers write a full obs (PMRL_OBS_FULL)");
+    return 0;
+}
+
+extern "C" int pmrl_rollout_gather_index_obs(int32_t S, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
+                                             const int32_t* slots, const int32_t* envs,
+                                             const int32_t* bi, const float* a, const float* v, const float* r,
+                                             const float* wp, const float* feat_am, const float* y_tm,
+                                             void* s_out, float* a_out, float* r_out, float* pv_out, float* pa_out, float* p_out,
+                                             int32_t obs_mode, void* stream) {
+    if (int rc = check_gather_obs_mode(obs_mode, F)) return rc;
+    return rollout_gather_index(S, E, A, W, F, T, B, slots, envs, bi, a, v, r, wp, feat_am, y_tm, s_out, a_out, r_out, pv_out,
+                                pa_out, p_out, (obs_mode & PMRL_OBS_BF16) != 0, obs_rel_of(obs_mode), stream);
+}
+
+extern "C" int pmrl_replay_gather_obs(int32_t P, int32_t L, int32_t E, int32_t A, int32_t W, int32_t F, int32_t T, int32_t B,
+                                      const int32_t* epochs, const int32_t* envs, const int32_t* starts,
+                                      const int32_t* bi, const float* ba, const float* br, const float* feat_am,
+                                      void* s_out, float* a_out, float* r_out, void* s2_out, int32_t obs_mode, void* stream) {
+    if (int rc = check_gather_obs_mode(obs_mode, F)) return rc;
+    return replay_gather(P, L, E, A, W, F, T, B, epochs, envs, starts, bi, ba, br, feat_am, s_out, a_out, r_out, s2_out,
+                         (obs_mode & PMRL_OBS_BF16) != 0, obs_rel_of(obs_mode), stream);
 }

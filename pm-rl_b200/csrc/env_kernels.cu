@@ -172,8 +172,9 @@ __global__ void __launch_bounds__(kStepThreads) k_env_reset(const StepParams p) 
 // Observation tiles from the current state.
 // ------------------------------------------------------------------------------------------------
 // OT: obs element type (float, or uint16_t bf16 bits — PMRL_OBS_BF16); the fp32 and bf16 kernels below share this body.
-template <typename OT>
-__device__ __forceinline__ void obs_build(const StepParams& p) {
+// REL: window-relative features (PMRL_OBS_REL, divisor channel / mask in rel).
+template <typename OT, bool REL = false>
+__device__ __forceinline__ void obs_build(const StepParams& p, const ObsRel& rel = ObsRel{0, 0u}) {
     extern __shared__ __align__(128) unsigned char smem_obs[];
     OT* const tile = reinterpret_cast<OT*>(smem_obs);
     const int e = blockIdx.x / p.tiles_per_env;
@@ -185,7 +186,7 @@ __device__ __forceinline__ void obs_build(const StepParams& p) {
     const int idx = p.idx[e], full = p.is_full[e];
     if (p.obs_mode == PMRL_OBS_FULL) {
         const int row0 = (p.t0 ? p.t0[e] : 0) + p.t[e];
-        obs_tile_fill_features(p, tile, a0, na, row0, tid, kObsThreads);
+        obs_tile_fill_features<OT, REL>(p, tile, a0, na, row0, tid, kObsThreads, rel);
     }
     obs_tile_fill_weights(p, tile, p.hist + (size_t)e * p.W * p.A, a0, na, idx, full, nullptr, -1, tid, kObsThreads);
     fence_proxy_async_smem();
@@ -195,6 +196,8 @@ __device__ __forceinline__ void obs_build(const StepParams& p) {
 }
 __global__ void __launch_bounds__(kObsThreads) k_obs_build(const StepParams p) { obs_build<float>(p); }
 __global__ void __launch_bounds__(kObsThreads) k_obs_build_bf16(const StepParams p) { obs_build<uint16_t>(p); }
+template <typename OT>
+__global__ void __launch_bounds__(kObsThreads) k_obs_build_rel(const StepParams p, const ObsRel rel) { obs_build<OT, true>(p, rel); }
 
 
 // The same tile for the common shape (4 feature channels + weight slot, W <= 64, 32-asset tiles), without the
@@ -260,10 +263,11 @@ __global__ void __launch_bounds__(kObsThreads) k_obs_build_rows(const StepParams
     }
 }
 
-// k_obs_build_rows with the tile in obs element type OT (instantiated for bf16 bits: k_obs_build_rows_bf16).  The fp32
-// kernel above keeps its own code: compiled through this template its SASS comes out reordered.
-template <typename OT>
-__device__ __forceinline__ void obs_build_rows(const StepParams& p) {
+// k_obs_build_rows with the tile in obs element type OT (instantiated for bf16 bits: k_obs_build_rows_bf16, and with REL for
+// both types: k_obs_build_rows_rel).  The fp32 kernel above keeps its own code: compiled through this template its SASS comes
+// out reordered.
+template <typename OT, bool REL = false>
+__device__ __forceinline__ void obs_build_rows(const StepParams& p, const ObsRel& rel = ObsRel{0, 0u}) {
     extern __shared__ __align__(128) unsigned char smem_obs[];
     OT* const tile = reinterpret_cast<OT*>(smem_obs);               // [32][W][5]
     const int A = p.A, W = p.W, T = p.T;
@@ -295,6 +299,11 @@ __device__ __forceinline__ void obs_build_rows(const StepParams& p) {
         const int w = warp + 8 * j, slot = w - shift;
         rv[j] = (w < W && slot >= 0 && lane < na) ? ld_once(ring + (size_t)slot * A, kPolicyEvictFirst) : 0.0f;
     }
+    if constexpr (REL) {              // window row W-1 sits in lane (W-1) & 31, chunk (W-1) >> 5 of the asset's warp
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+            if (warp + 8 * i < na) rel_divide_staged<2, 1>(fv[i], (unsigned)w0 | ((unsigned)w1 << 1), (W - 1) & 31, (W - 1) >> 5, rel);
+    }
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         const int al = warp + 8 * i;
@@ -323,6 +332,8 @@ __device__ __forceinline__ void obs_build_rows(const StepParams& p) {
 }
 
 __global__ void __launch_bounds__(kObsThreads) k_obs_build_rows_bf16(const StepParams p) { obs_build_rows<uint16_t>(p); }
+template <typename OT>
+__global__ void __launch_bounds__(kObsThreads) k_obs_build_rows_rel(const StepParams p, const ObsRel rel) { obs_build_rows<OT, true>(p, rel); }
 
 }  // namespace pmrl
 
@@ -377,10 +388,11 @@ static int fill_params(const PmrlEnvCfg* cfg, const PmrlTables* tbl, const PmrlE
     return 0;
 }
 
-// obs_mode as passed by the caller (PMRL_OBS_BF16 included); the rest of the library works with the base mode and a bf16 flag
+// obs_mode as passed by the caller (PMRL_OBS_BF16 / PMRL_OBS_REL bits included); the rest of the library works with the base
+// mode, a bf16 flag and the ObsRel of obs_rel_of
 static int check_obs_args(const StepParams& p, const float* obs, int obs_mode_arg) {
-    if (int rc = pmrl_check_obs_mode(obs_mode_arg)) return rc;
-    const int obs_mode = obs_mode_arg & ~PMRL_OBS_BF16;
+    if (int rc = pmrl_check_obs_mode(obs_mode_arg, p.F)) return rc;
+    const int obs_mode = obs_mode_arg & 0xFF;
     if (obs_mode == PMRL_OBS_NONE) return 0;
     if (!obs) return pmrl_fail(PMRL_E_ARG, "obs is NULL but obs_mode != NONE");
     if (p.F < 2 && obs_mode == PMRL_OBS_FULL) return pmrl_fail(PMRL_E_SHAPE, "F >= 2 required for a full obs");
@@ -399,8 +411,9 @@ static int check_obs_args(const StepParams& p, const float* obs, int obs_mode_ar
 // Launch-shape knobs (pmrl_set_tuning).
 static int g_tune_group = 0, g_tune_ctas_per_sm = 0, g_tune_fused = 1, g_tune_fast = 1, g_tune_rt = 1;
 
-// obs_mode: base mode (FULL / WEIGHTS); bf16: PMRL_OBS_BF16 was set (FULL only, checked by check_obs_args)
-static int launch_obs(StepParams& p, float* obs, int obs_mode, bool bf16, cudaStream_t s) {
+// obs_mode: base mode (FULL / WEIGHTS); bf16: PMRL_OBS_BF16 was set; rel: PMRL_OBS_REL's channels (mask 0: off); both FULL only,
+// checked by check_obs_args
+static int launch_obs(StepParams& p, float* obs, int obs_mode, bool bf16, const ObsRel& rel, cudaStream_t s) {
     p.obs = obs; p.obs_mode = obs_mode;
     const size_t esz = bf16 ? 2 : 4;
     if (obs_mode == PMRL_OBS_FULL && p.F == 5 && p.W <= 64 && p.t0 && g_tune_fast) {      // division-free tile kernel
@@ -409,6 +422,11 @@ static int launch_obs(StepParams& p, float* obs, int obs_mode, bool bf16, cudaSt
         p.tiles_per_env = (p.A + 31) / 32;
         const long grid = (long)p.E * p.tiles_per_env;
         if (grid > 2147483647L) return pmrl_fail(PMRL_E_SHAPE, "E * tiles_per_env exceeds the grid limit");
+        if (rel.mask) {
+            if (bf16) k_obs_build_rows_rel<uint16_t><<<(unsigned)grid, kObsThreads, (size_t)32 * p.W * 5 * esz, s>>>(p, rel);
+            else k_obs_build_rows_rel<float><<<(unsigned)grid, kObsThreads, (size_t)32 * p.W * 5 * esz, s>>>(p, rel);
+            return pmrl_check_launch(bf16 ? "k_obs_build_rows_rel<bf16>" : "k_obs_build_rows_rel<float>");
+        }
         if (bf16) {
             k_obs_build_rows_bf16<<<(unsigned)grid, kObsThreads, (size_t)32 * p.W * 5 * esz, s>>>(p);
             return pmrl_check_launch("k_obs_build_rows_bf16");
@@ -421,6 +439,11 @@ static int launch_obs(StepParams& p, float* obs, int obs_mode, bool bf16, cudaSt
     const size_t smem = (size_t)p.tile_assets * p.W * p.F * esz;
     const long grid = (long)p.E * p.tiles_per_env;
     if (grid > 2147483647L) return pmrl_fail(PMRL_E_SHAPE, "E * tiles_per_env exceeds the grid limit");
+    if (rel.mask) {
+        if (bf16) k_obs_build_rel<uint16_t><<<(unsigned)grid, kObsThreads, smem, s>>>(p, rel);
+        else k_obs_build_rel<float><<<(unsigned)grid, kObsThreads, smem, s>>>(p, rel);
+        return pmrl_check_launch(bf16 ? "k_obs_build_rel<bf16>" : "k_obs_build_rel<float>");
+    }
     if (bf16) {
         k_obs_build_bf16<<<(unsigned)grid, kObsThreads, smem, s>>>(p);
         return pmrl_check_launch("k_obs_build_bf16");
@@ -510,15 +533,15 @@ extern "C" int pmrl_set_tuning(int32_t key, int32_t value) {
     }
 }
 
-static int launch_fused(StepParams& p, float* obs, int npl, int vec, bool bf16, cudaStream_t s) {
+static int launch_fused(StepParams& p, float* obs, int npl, int vec, bool bf16, const ObsRel& rel, cudaStream_t s) {
     p.obs = obs; p.obs_mode = PMRL_OBS_FULL;
     if (!g_tune_fast) return -100;
     if (g_tune_rt) {                                  // ring rows through one TMA bulk load per env (env_step_rt.cu)
         p.prefetch_next = (g_tune_rt == 2) ? 0 : 1;
-        const int rc = pmrl_launch_step_obs_rt(p, npl, vec, g_tune_group, g_tune_ctas_per_sm, bf16, s);
+        const int rc = pmrl_launch_step_obs_rt(p, npl, vec, g_tune_group, g_tune_ctas_per_sm, bf16, rel, s);
         if (rc != -100) return rc;
     }
-    if (bf16) return -100;                            // no bf16 form of the register-staged kernel: its shapes take the two kernels
+    if (bf16 || rel.mask) return -100;                // no bf16 or REL form of the register-staged kernel: its shapes take the two kernels
     // register-staged fill (env_step_fast.cu): F == 5, W <= 64, A <= 128 — the shapes RT's ring alignment excludes
     return pmrl_launch_step_obs_fast(p, npl, vec, g_tune_group, g_tune_ctas_per_sm, s);
     // -100: no fused kernel covers this shape (A > 128, F != 5, W > 64) → state-only step, then the obs tile kernel
@@ -536,7 +559,7 @@ extern "C" int pmrl_env_reset(const PmrlEnvCfg* cfg, const PmrlTables* tbl, cons
     const int cap = pmrl_sm_count() * 8;
     k_env_reset<<<want < cap ? want : cap, kStepThreads, 0, s>>>(p);
     if (int rc = pmrl_check_launch("k_env_reset")) return rc;
-    if (obs_mode != PMRL_OBS_NONE) return launch_obs(p, obs, obs_mode & ~PMRL_OBS_BF16, (obs_mode & PMRL_OBS_BF16) != 0, s);
+    if (obs_mode != PMRL_OBS_NONE) return launch_obs(p, obs, obs_mode & 0xFF, (obs_mode & PMRL_OBS_BF16) != 0, obs_rel_of(obs_mode), s);
     return 0;
 }
 
@@ -593,7 +616,7 @@ extern "C" int pmrl_obs_build(const PmrlEnvCfg* cfg, const PmrlTables* tbl, cons
     if (int rc = fill_params(cfg, tbl, st, p)) return rc;
     if (obs_mode == PMRL_OBS_NONE) return pmrl_fail(PMRL_E_ARG, "obs_mode NONE makes no obs");
     if (int rc = check_obs_args(p, obs, obs_mode)) return rc;
-    return launch_obs(p, obs, obs_mode & ~PMRL_OBS_BF16, (obs_mode & PMRL_OBS_BF16) != 0, (cudaStream_t)stream);
+    return launch_obs(p, obs, obs_mode & 0xFF, (obs_mode & PMRL_OBS_BF16) != 0, obs_rel_of(obs_mode), (cudaStream_t)stream);
 }
 
 // validation shared by the step entry points; fills the per-step fields of p
@@ -639,16 +662,17 @@ extern "C" int pmrl_env_step_io(const PmrlEnvCfg* cfg, const PmrlTables* tbl, co
     if (int rc = prepare_step(cfg, tbl, st, io, p)) return rc;
     float* obs = io->obs;
     if (int rc = check_obs_args(p, obs, io->obs_mode)) return rc;
-    const int obs_mode = io->obs_mode & ~PMRL_OBS_BF16;
+    const int obs_mode = io->obs_mode & 0xFF;
     const bool bf16 = (io->obs_mode & PMRL_OBS_BF16) != 0;
+    const ObsRel rel = obs_rel_of(io->obs_mode);
     const int npl = env_npl_for(p.A), vec = vec_for_pointers(p, npl);
     cudaStream_t s = (cudaStream_t)stream;
     if (obs_mode == PMRL_OBS_FULL && g_tune_fused && (size_t)p.W * p.F * 4 <= 36 * 1024) {
-        const int rc = launch_fused(p, obs, npl, vec, bf16, s);
+        const int rc = launch_fused(p, obs, npl, vec, bf16, rel, s);
         if (rc != -100) return rc;                    // -100: no fused kernel for this shape → step kernel + obs kernel
     }
     if (int rc = launch_step_s(p, npl, vec, s)) return rc;
-    if (obs_mode != PMRL_OBS_NONE) return launch_obs(p, obs, obs_mode, bf16, s);
+    if (obs_mode != PMRL_OBS_NONE) return launch_obs(p, obs, obs_mode, bf16, rel, s);
     return 0;
 }
 

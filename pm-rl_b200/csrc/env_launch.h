@@ -4,8 +4,10 @@
 #include "pmrl_device.cuh"
 
 // Fused step+obs kernel whose weight rings enter shared memory as one TMA bulk load per env (env_step_rt.cu).
-// bf16: obs as bf16 bit patterns (PMRL_OBS_BF16).  Returns -100 if the shape is not covered by this kernel (caller falls back).
-int pmrl_launch_step_obs_rt(pmrl::StepParams& p, int npl, int vec, int group, int ctas_per_sm, bool bf16, cudaStream_t s);
+// bf16: obs as bf16 bit patterns (PMRL_OBS_BF16); rel: window-relative features (PMRL_OBS_REL; mask 0 = off).  Returns -100 if
+// the shape is not covered by this kernel (caller falls back).
+int pmrl_launch_step_obs_rt(pmrl::StepParams& p, int npl, int vec, int group, int ctas_per_sm, bool bf16, const pmrl::ObsRel& rel,
+                            cudaStream_t s);
 
 // Register-staged fused step+obs kernel (env_step_fast.cu).  Returns -100 if the shape is not covered.
 int pmrl_launch_step_obs_fast(pmrl::StepParams& p, int npl, int vec, int group, int ctas_per_sm, cudaStream_t s);

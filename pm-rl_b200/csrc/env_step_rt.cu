@@ -325,9 +325,12 @@ __global__ void __launch_bounds__(kRtThreads, 2) k_env_step_obs_rt(const StepPar
 // instantiated for bf16 only.  The fp32 kernel keeps its own copy: routing it through this template compiles to different
 // (reordered, re-allocated) SASS for all 108 fp32 instantiations, and the fp32 path is the measured, pinned reference.
 // (#128 "loop is not reachable": with W = 50 compiled in, the bf16 paired-row fill `continue`s past the generic one)
+// REL (k_env_step_obs_rt_rel, fp32 and bf16, PAD = false): window-relative features (PMRL_OBS_REL), the staged chunks of a tile
+// divided in registers just before they are spilled to shared memory (rel_divide_staged).
 #pragma nv_diag_suppress 128
-template <typename OT, int NPL, bool HASC, int VEC, int WT, int C4, bool PAD>
-__device__ __forceinline__ void env_step_obs_rt(const StepParams& p) {
+template <typename OT, int NPL, bool HASC, int VEC, int WT, int C4, bool PAD, bool REL = false>
+__device__ __forceinline__ void env_step_obs_rt(const StepParams& p, const ObsRel& rel = ObsRel{0, 0u}) {
+    static_assert(!(REL && PAD), "no REL form of the channel-padded instantiations");
     constexpr bool BF = sizeof(OT) == 2;
     using Geo = RtGeom<C4>;
     using Feat = RtFeat<C4, WT>;
@@ -491,6 +494,22 @@ __device__ __forceinline__ void env_step_obs_rt(const StepParams& p) {
                 }
             }
         };
+        // REL: the divisor is window row W-1 of each staged asset row — lane (W-1) & 31, chunk (W-1) >> 5 (paired bf16 rows:
+        // lane W/2 - 1, its second row)
+        [[maybe_unused]] auto rel_feat = [&](Feat& fr, int r0, auto partial) {
+            constexpr bool PARTIAL = decltype(partial)::value;
+            const int nr = PARTIAL ? R - r0 : TR;
+            unsigned held = 0u;
+            int src_lane = (W - 1) & 31, src_m = ((W - 1) >> 5) * C4 + (rel.ref >> 2);
+#pragma unroll
+            for (int m = 0; m < MW; ++m) held |= (unsigned)(lane + 32 * (m / C4) < W) << m;
+            if constexpr (BF && C4 == 1 && !PAD) {
+                if (pair) { held = 2 * lane < W ? 3u : 0u; src_lane = (W >> 1) - 1; src_m = 1; }
+            }
+#pragma unroll
+            for (int i = 0; i < RPW; ++i)
+                if (!PARTIAL || warp + 8 * i < nr) rel_divide_staged<MW, C4>(fr.fv[i], held, src_lane, src_m, rel);
+        };
         auto spill_tile = [&](const Feat& fr, OT* __restrict__ tile, int r0, auto partial) {
             constexpr bool PARTIAL = decltype(partial)::value;
             const int nr = PARTIAL ? R - r0 : TR;
@@ -574,6 +593,9 @@ __device__ __forceinline__ void env_step_obs_rt(const StepParams& p) {
             // for exactly this hand-over; barrier stalls were the largest stall reason, 2.0 per issue at F = 5, 2.8 at F = 9.)
             OT* const tile = buf ? tile1 : tile0;
             const int r0 = ti * TR;
+            if constexpr (REL) {
+                if (ti < nfull) rel_feat(fr, r0, std::false_type{}); else rel_feat(fr, r0, std::true_type{});
+            }
             if (ti < nfull) spill_tile(fr, tile, r0, std::false_type{}); else spill_tile(fr, tile, r0, std::true_type{});
             if (ti + 1 < ntiles) {
                 if (ti + 1 < nfull) load_feat(fr, r0 + TR, std::false_type{}); else load_feat(fr, r0 + TR, std::true_type{});
@@ -613,32 +635,54 @@ template <int NPL, bool HASC, int VEC, int WT, int C4, bool PAD = false>
 __global__ void __launch_bounds__(kRtThreads, 2) k_env_step_obs_rt_bf16(const StepParams p) {
     env_step_obs_rt<uint16_t, NPL, HASC, VEC, WT, C4, PAD>(p);
 }
+template <typename OT, int NPL, bool HASC, int VEC, int WT, int C4>
+__global__ void __launch_bounds__(kRtThreads, 2) k_env_step_obs_rt_rel(const StepParams p, const ObsRel rel) {
+    env_step_obs_rt<OT, NPL, HASC, VEC, WT, C4, false, true>(p, rel);
+}
 
 }  // namespace pmrl
 
 using namespace pmrl;
 
-template <bool BF, int NPL, bool HASC, int VEC, int WT, int C4, bool PAD>
-static int launch_rt_t(StepParams& p, size_t smem, int grid, cudaStream_t s) {
-    constexpr auto kernel = BF ? k_env_step_obs_rt_bf16<NPL, HASC, VEC, WT, C4, PAD> : k_env_step_obs_rt<NPL, HASC, VEC, WT, C4, PAD>;
-    const char* const name = BF ? "k_env_step_obs_rt_bf16" : "k_env_step_obs_rt";
-    static bool attr_done[64] = {false};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev >= 0 && dev < 64 && !attr_done[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024);
-        if (e != cudaSuccess) return pmrl_fail((int)e, BF ? "cudaFuncSetAttribute(k_env_step_obs_rt_bf16) failed" : "cudaFuncSetAttribute(k_env_step_obs_rt) failed");
-        attr_done[dev] = true;
+// REL kernels take the ObsRel as a second parameter
+template <bool BF, bool REL, int NPL, bool HASC, int VEC, int WT, int C4, bool PAD>
+static int launch_rt_t(StepParams& p, const ObsRel& rel, size_t smem, int grid, cudaStream_t s) {
+    if constexpr (REL) {
+        using OT = std::conditional_t<BF, uint16_t, float>;
+        constexpr auto kernel = k_env_step_obs_rt_rel<OT, NPL, HASC, VEC, WT, C4>;
+        static bool attr_done[64] = {false};
+        int dev = 0;
+        cudaGetDevice(&dev);
+        if (dev >= 0 && dev < 64 && !attr_done[dev]) {
+            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024);
+            if (e != cudaSuccess) return pmrl_fail((int)e, "cudaFuncSetAttribute(k_env_step_obs_rt_rel) failed");
+            attr_done[dev] = true;
+        }
+        kernel<<<grid, kRtThreads, smem, s>>>(p, rel);
+        return pmrl_check_launch(BF ? "k_env_step_obs_rt_rel<bf16>" : "k_env_step_obs_rt_rel<float>");
+    } else {
+        constexpr auto kernel = BF ? k_env_step_obs_rt_bf16<NPL, HASC, VEC, WT, C4, PAD> : k_env_step_obs_rt<NPL, HASC, VEC, WT, C4, PAD>;
+        const char* const name = BF ? "k_env_step_obs_rt_bf16" : "k_env_step_obs_rt";
+        static bool attr_done[64] = {false};
+        int dev = 0;
+        cudaGetDevice(&dev);
+        if (dev >= 0 && dev < 64 && !attr_done[dev]) {
+            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024);
+            if (e != cudaSuccess) return pmrl_fail((int)e, BF ? "cudaFuncSetAttribute(k_env_step_obs_rt_bf16) failed" : "cudaFuncSetAttribute(k_env_step_obs_rt) failed");
+            attr_done[dev] = true;
+        }
+        kernel<<<grid, kRtThreads, smem, s>>>(p);
+        return pmrl_check_launch(name);
     }
-    kernel<<<grid, kRtThreads, smem, s>>>(p);
-    return pmrl_check_launch(name);
 }
 
-template <bool BF, int NPL, int VEC, int C4, bool PAD>
-static int launch_rt_w(StepParams& p, size_t smem, int grid, cudaStream_t s) {
+template <bool BF, bool REL, int NPL, int VEC, int C4, bool PAD>
+static int launch_rt_w(StepParams& p, const ObsRel& rel, size_t smem, int grid, cudaStream_t s) {
     const bool hasc = p.commission > 0.0f;
-    if (p.W == 50) return hasc ? launch_rt_t<BF, NPL, true, VEC, 50, C4, PAD>(p, smem, grid, s) : launch_rt_t<BF, NPL, false, VEC, 50, C4, PAD>(p, smem, grid, s);
-    return hasc ? launch_rt_t<BF, NPL, true, VEC, 0, C4, PAD>(p, smem, grid, s) : launch_rt_t<BF, NPL, false, VEC, 0, C4, PAD>(p, smem, grid, s);
+    if (p.W == 50) return hasc ? launch_rt_t<BF, REL, NPL, true, VEC, 50, C4, PAD>(p, rel, smem, grid, s)
+                               : launch_rt_t<BF, REL, NPL, false, VEC, 50, C4, PAD>(p, rel, smem, grid, s);
+    return hasc ? launch_rt_t<BF, REL, NPL, true, VEC, 0, C4, PAD>(p, rel, smem, grid, s)
+                : launch_rt_t<BF, REL, NPL, false, VEC, 0, C4, PAD>(p, rel, smem, grid, s);
 }
 
 // Envs per group for a batch of E envs on `slots` persistent CTAs.  A CTA's time is (rounds it runs) x (envs per group +
@@ -659,7 +703,7 @@ static int pick_group(int E, int slots, int gmax, int step) {
     return best;
 }
 
-int pmrl_launch_step_obs_rt(StepParams& p, int npl, int vec, int group, int ctas_per_sm, bool bf16, cudaStream_t s) {
+int pmrl_launch_step_obs_rt(StepParams& p, int npl, int vec, int group, int ctas_per_sm, bool bf16, const ObsRel& rel, cudaStream_t s) {
     // four feature channels per float4 chunk of the asset-major table: F = 5, 9, 13, 17 read feat_am directly, every other
     // F in [2, 17] needs the channel-padded copy feat_am4
     if (p.F < 2 || p.F > 17) return -100;
@@ -693,10 +737,19 @@ int pmrl_launch_step_obs_rt(StepParams& p, int npl, int vec, int group, int ctas
     const int n_groups = (p.E + G - 1) / G;
     const int grid = n_groups < slots ? n_groups : slots;
     const bool pad = (p.F - 1) % 4 != 0;
+    if (rel.mask) {
+        // window-relative obs: F = 5 and 9 (the OHLC and OHLC + indicator tables); every other width takes the two kernels
+#define RT_REL(N, V, C) if (npl == N && vec == V && c4 == C && !pad) \
+        return bf16 ? launch_rt_w<true, true, N, V, C, false>(p, rel, smem, grid, s) : launch_rt_w<false, true, N, V, C, false>(p, rel, smem, grid, s)
+        RT_REL(1, 1, 1); RT_REL(2, 1, 1); RT_REL(2, 2, 1); RT_REL(4, 1, 1); RT_REL(4, 2, 1); RT_REL(4, 4, 1);
+        RT_REL(2, 2, 2); RT_REL(4, 2, 2); RT_REL(4, 4, 2);
+#undef RT_REL
+        return -100;
+    }
 #define RT_CASE(N, V, C) if (npl == N && vec == V && c4 == C && !pad) \
-        return bf16 ? launch_rt_w<true, N, V, C, false>(p, smem, grid, s) : launch_rt_w<false, N, V, C, false>(p, smem, grid, s)
+        return bf16 ? launch_rt_w<true, false, N, V, C, false>(p, rel, smem, grid, s) : launch_rt_w<false, false, N, V, C, false>(p, rel, smem, grid, s)
 #define RT_PAD(N, V, C) if (npl == N && vec == V && c4 == C && pad) \
-        return bf16 ? launch_rt_w<true, N, V, C, true>(p, smem, grid, s) : launch_rt_w<false, N, V, C, true>(p, smem, grid, s)
+        return bf16 ? launch_rt_w<true, false, N, V, C, true>(p, rel, smem, grid, s) : launch_rt_w<false, false, N, V, C, true>(p, rel, smem, grid, s)
     RT_CASE(1, 1, 1); RT_CASE(2, 1, 1); RT_CASE(2, 2, 1); RT_CASE(4, 1, 1); RT_CASE(4, 2, 1); RT_CASE(4, 4, 1);
     // wider feature sets and padded tables: the even / 16-byte asset maps only (odd asset counts take the two-kernel path)
     RT_CASE(2, 2, 2); RT_CASE(4, 2, 2); RT_CASE(4, 4, 2);

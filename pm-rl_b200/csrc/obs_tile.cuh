@@ -13,10 +13,12 @@
 
 namespace pmrl {
 
-// Feature channels 0..F-2 of the tile from the asset-major table (rows row0 .. row0+W-1).
-template <typename OT>
+// Feature channels 0..F-2 of the tile from the asset-major table (rows row0 .. row0+W-1).  REL (PMRL_OBS_REL): the channels
+// in rel.mask are divided by channel rel.ref of row row0+W-1 of their asset (rel_quot: the bits of IEEE division).
+template <typename OT, bool REL = false>
 __device__ __forceinline__ void obs_tile_fill_features(const StepParams& p, OT* __restrict__ tile,
-                                                       int a0, int na, int row0, int tid, int nthreads) {
+                                                       int a0, int na, int row0, int tid, int nthreads,
+                                                       const ObsRel& rel = ObsRel{0, 0u}) {
     const int W = p.W, F = p.F, Fm1 = p.F - 1, T = p.T;
     const uint64_t pol_keep = l2_policy_evict_last();
     if (Fm1 == 4) {
@@ -26,7 +28,16 @@ __device__ __forceinline__ void obs_tile_fill_features(const StepParams& p, OT* 
         const int n = na * W;
         for (int r = tid; r < n; r += nthreads) {
             const int al = r / W, w = r - al * W;
-            const float4 v = ld_keep4(tbl + (size_t)(a0 + al) * T + row0 + w, pol_keep);
+            float4 v = ld_keep4(tbl + (size_t)(a0 + al) * T + row0 + w, pol_keep);
+            if constexpr (REL) {        // the divisor row: the same 16 bytes for the W threads of one asset (L1 hits)
+                const float b = f4_get(ld_keep4(tbl + (size_t)(a0 + al) * T + row0 + W - 1, pol_keep), rel.ref);
+                const bool b_ok = unidiv_in_range(b);
+                const UniDiv dv = unidiv_make(b);
+                if (rel.mask & 1u) v.x = rel_quot(v.x, b, dv, b_ok);
+                if (rel.mask & 2u) v.y = rel_quot(v.y, b, dv, b_ok);
+                if (rel.mask & 4u) v.z = rel_quot(v.z, b, dv, b_ok);
+                if (rel.mask & 8u) v.w = rel_quot(v.w, b, dv, b_ok);
+            }
             OT* d = tile + r * 5;
             d[0] = obs_cvt<OT>(v.x); d[1] = obs_cvt<OT>(v.y); d[2] = obs_cvt<OT>(v.z); d[3] = obs_cvt<OT>(v.w);
         }
@@ -41,9 +52,19 @@ __device__ __forceinline__ void obs_tile_fill_features(const StepParams& p, OT* 
         for (int al = warp; al < na; al += nwarps) {
             const float* __restrict__ src = p.feat_am + ((size_t)(a0 + al) * T + row0) * Fm1;
             OT* __restrict__ drow = tile + al * W * F;
+            float b = 0.0f;
+            bool b_ok = false;
+            UniDiv dv = {0.0f, 0.0f};
+            if constexpr (REL) {        // one broadcast load of the divisor per asset row
+                b = ld_keep(src + (W - 1) * Fm1 + rel.ref, pol_keep);
+                b_ok = unidiv_in_range(b);
+                dv = unidiv_make(b);
+            }
             int w = w_first, c = c_first;
             for (int rem = lane; rem < per_asset; rem += 32) {
-                drow[w * F + c] = obs_cvt<OT>(ld_keep(src + rem, pol_keep));
+                float x = ld_keep(src + rem, pol_keep);
+                if constexpr (REL) { if ((rel.mask >> c) & 1u) x = rel_quot(x, b, dv, b_ok); }
+                drow[w * F + c] = obs_cvt<OT>(x);
                 w += dq; c += dr;
                 if (c >= Fm1) { c -= Fm1; ++w; }
             }

@@ -46,6 +46,10 @@ class BatchedTradingEnv:
     With `cfg.obs_dtype == "bfloat16"` every obs this env returns or writes (`reset`, `step`, `step_io`, `step_host`,
     `graphed_step`, `observe`, and `out=` buffers, which must then be bfloat16) is the bf16 rounding of the fp32 obs;
     state, rewards and the buffer rows written through `step_io` stay fp32.
+
+    With `cfg.obs_relative_to = ref` the same obs are window-relative: channel c in `cfg.obs_relative_channels` of every
+    asset's window is divided (IEEE fp32 division) by channel `ref` of that window's last row, inside the obs kernels;
+    the weight channel, state and rewards are unchanged.
     """
 
     @classmethod
@@ -64,7 +68,8 @@ class BatchedTradingEnv:
         E, A, W, F = cfg.num_envs, cfg.num_assets, cfg.window_size, cfg.num_features
         self.E, self.A, self.W, self.F = E, A, W, F
         self.obs_dtype = OBS_TORCH_DTYPES[cfg.obs_dtype]
-        self._obs_full = OBS_FULL | (OBS_BF16 if self.obs_dtype is torch.bfloat16 else 0)   # obs_mode of every obs this env makes
+        # obs_mode of every obs this env makes
+        self._obs_full = OBS_FULL | (OBS_BF16 if self.obs_dtype is torch.bfloat16 else 0) | cfg.obs_relative_bits
         dev = self.device
         self.close_tm = None
         self.feat_am = None

@@ -12,6 +12,18 @@ from __future__ import annotations
 import torch
 
 
+def _check_relative(env, buffer):
+    """A buffer that regenerates windows (index-mode rollout, replay) must divide them like the env does."""
+    if buffer is None or getattr(buffer, "mode", "index") == "full":
+        return
+    want = (env.cfg.obs_relative_to, env.cfg.obs_relative_channels)
+    got = (buffer.obs_relative_to, buffer.obs_relative_channels)
+    if want != got:
+        raise ValueError(f"the buffer regenerates windows with obs_relative_to / obs_relative_channels = {got}, the env makes "
+                         f"them with {want}: a sample would not equal the obs the env returned; build the buffer with the "
+                         "env config's settings")
+
+
 @torch.no_grad()
 def collect_on_policy(env, act_fn, buffer, num_items: int):
     """env: BatchedTradingEnv; act_fn(obs [E,A,W,F]) -> actions [E,A(,1)]; buffer: DeviceRolloutBuffer or None.
@@ -20,6 +32,7 @@ def collect_on_policy(env, act_fn, buffer, num_items: int):
     The step kernel writes the buffer rows itself (`buffer.sinks`): reward, raw action and post-step value of item k go
     to slot k - (W-1), and the obs the step returns — the obs stored WITH the next item (on_policy.py:65 stores the obs
     before the step) — is materialised directly in s[slot + 1].  No copy kernel, no second obs pass, no host sync."""
+    _check_relative(env, buffer)
     if buffer is not None:
         buffer.reset()
     s = env.reset()
@@ -38,6 +51,7 @@ def collect_off_policy(env, act_fn, buffer, epoch: int, num_items: int):
     """env: BatchedTradingEnv; buffer: DeviceReplayBuffer.  `buffer.add(epoch, step, a, r)` per item (off_policy.py:87),
     with the (i, a, r) row written by the step kernel: `i` is each env's OWN loader index t0[e] + k — the row the replay
     gather regenerates s and s' from (buffer.py:65-68) — not the lockstep counter."""
+    _check_relative(env, buffer)
     s = env.reset()
     for step in range(1, num_items):
         a = act_fn(s)
